@@ -3,7 +3,8 @@
 and MCL iterations/sec, on the synthetic 50k-contig / 200M-pair workload (BASELINE.json configs[2]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
-    python bench.py --impl reference [...]                          # the UNMODIFIED reference (baseline/_ref) on the host cores
+    python bench.py --impl reference [...]                          # the UNMODIFIED reference (oracle/_ref) on the host cores
+    python bench.py --dump-outputs DIR [...]                        # also write the last timed step's outputs as DIR/*.npy
 
 One "step" = one pass of the hot path over the whole synthetic input:
     link counting (200M records) -> first-seen index -> symmetric CSC -> column normalise ->
@@ -31,6 +32,8 @@ if REPO not in sys.path:
 
 import numpy as np
 
+REF_MISSING = "the unmodified reference is not built into oracle/_ref (__graft_entry__.build() with a HapHiC checkout)"
+
 
 def parse_args():
     p = argparse.ArgumentParser()
@@ -54,7 +57,15 @@ def parse_args():
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--no-default-sweep", action="store_true", help="skip the 20-inflation default sweep figure")
     p.add_argument("--verbose", action="store_true")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="write what the last timed step computed as DIR/<name>.npy (float64, seeded samples of the large "
+                        "arrays, at most 64 MB in all), so that two builds can be compared output for output")
+    a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "b200":
+        p.error("--dump-outputs applies to --impl b200")
+    return a
 
 
 def workload_name(a):
@@ -117,14 +128,18 @@ def cpu_baseline_block(a, asm, rank, in_nx, rec):
     """CPU legs on this box's host cores, bounded samples of the same stream: the unmodified reference's pair loop
     (kind "reference"), and beside it the single-core C port of the same loop (oracle/haphic_oracle.c)."""
     import tempfile
-    n_ref = min(int(rec.shape[0]), a.cpu_sample_pairs)
-    sample = rec[:n_ref].cpu().numpy()
-    with tempfile.TemporaryDirectory() as tmp:
-        v, dt, nnz = ref_pairs_per_sec(asm, sample, tmp)
-    cpu = {"value": v, "unit": "pairs/s", "cores": 1, "kind": "reference",
-           "sample": "first {} records as .pairs text through the unmodified HapHiC_cluster.parse_alignments_for_ctgs("
-                     "pairs_generator_inter_ctgs(...)) from baseline/_ref, {:.1f} s (single-threaded Python by construction; "
-                     "host has {} cores)".format(len(sample), dt, os.cpu_count())}
+    from oracle import refimpl
+    if refimpl.available():
+        n_ref = min(int(rec.shape[0]), a.cpu_sample_pairs)
+        sample = rec[:n_ref].cpu().numpy()
+        with tempfile.TemporaryDirectory() as tmp:
+            v, dt, nnz = ref_pairs_per_sec(asm, sample, tmp)
+        cpu = {"value": v, "unit": "pairs/s", "cores": 1, "kind": "reference",
+               "sample": "first {} records as .pairs text through the unmodified HapHiC_cluster.parse_alignments_for_ctgs("
+                         "pairs_generator_inter_ctgs(...)) from oracle/_ref, {:.1f} s (single-threaded Python by construction; "
+                         "host has {} cores)".format(len(sample), dt, os.cpu_count())}
+    else:
+        cpu = {"unavailable": REF_MISSING}
     try:
         big = rec[: 8_000_000].cpu().numpy()
         vc, dtc = cpu_c_pairs_per_sec(asm, rank, in_nx, big)
@@ -196,7 +211,7 @@ def cpu_pairs_per_sec(asm, rank, in_nx, sample):
 
 
 def ref_pairs_per_sec(asm, sample, tmp):
-    """The reference's OWN per-read-pair loop, unmodified (baseline/_ref/HapHiC_cluster.py imported by oracle/refimpl.py):
+    """The reference's OWN per-read-pair loop, unmodified (oracle/_ref/HapHiC_cluster imported by oracle/refimpl.py):
     parse_alignments_for_ctgs over pairs_generator_inter_ctgs on a .pairs text of the sample (1562-1583, 1596-1655),
     single-threaded by construction.  Returns (pairs/s, seconds, distinct pairs)."""
     from oracle import refimpl
@@ -305,6 +320,58 @@ def make_inputs(a, device, rank_id=0, world=1):
     return asm, rank, in_nx, rec, lo
 
 
+# --------------------------------------------------------------------------------------------------
+# --dump-outputs: the arrays a caller of the timed path receives, as float64 (exact for every integer here)
+# --------------------------------------------------------------------------------------------------
+
+DUMP_ROWS = 1 << 18           # rows kept of the link table and of the link matrix
+DUMP_MCL_ROWS = 1 << 20       # entries kept of the final MCL matrices, shared by the inflations
+DUMP_LIMIT = 64 << 20         # bytes over all files
+
+
+def sample_index(n, cap, seed):
+    """0 .. n-1, or `cap` of them drawn with a fixed seed, ascending: the same positions for the same n in every run."""
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, size=cap, replace=False))
+
+
+def csc_sample(m, cap, seed):
+    """[k, 3] (row, column, value) of the stored entries of a scipy CSC matrix, all or a seeded sample, in storage order."""
+    k = sample_index(m.nnz, cap, seed)
+    col = np.searchsorted(m.indptr, k, side="right") - 1
+    return np.stack([m.indices[k].astype(np.float64), col.astype(np.float64), m.data[k].astype(np.float64)], axis=1)
+
+
+def dump_mcl_result(dump, inflation, st, result, cap):
+    name = "mcl_inflation_{}".format(inflation)
+    dump[name] = csc_sample(result, cap, 3)
+    dump[name + "_iterations"] = np.stack([st["iter_nnz"], st["iter_delta"]], axis=1)        # nnz and delta per round
+    dump.setdefault("mcl_summary", []).append([inflation, st["rounds"], st["converged"], result.nnz])
+
+
+def dump_links(dump, tab, info, index, n_linked, mat, mc):
+    f = tab.fetch()
+    k = sample_index(int(info.nnz_full), DUMP_ROWS, 1)
+    # full_link_dict entries in insertion order: key_i, key_j, full, flank, first_full, first_flank, HH, HT, TH, TT
+    dump["links"] = np.column_stack([f[c][k].astype(np.float64) for c in ("key_i", "key_j", "full", "flank", "first_full",
+                                                                          "first_flank")] + [f["ht"][k].astype(np.float64)])
+    dump["ctg_links"] = tab.fetch_ctg()
+    dump["matrix_index"] = index
+    dump["matrix"] = csc_sample(mat.to_scipy(), DUMP_ROWS, 2)
+    dump["counts"] = [info.n_records, info.n_used, info.nnz_full, info.nnz_flank, n_linked, mat.n, mat.nnz, mc.nnz_m0]
+
+
+def write_dump(path, dump):
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in dump.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("--dump-outputs: {} bytes exceed the limit of {}".format(total, DUMP_LIMIT))
+    os.makedirs(path, exist_ok=True)
+    for k, v in sorted(arrays.items()):
+        np.save(os.path.join(path, k + ".npy"), v)
+
+
 def run_reference(a):
     """`--impl reference`: the unmodified reference's hot loops on the host cores, bounded samples of the same workload."""
     rank_id = int(os.environ.get("RANK", "0"))
@@ -314,8 +381,7 @@ def run_reference(a):
     from haphic_b200 import synth
     from oracle import refimpl
     if not refimpl.available():
-        print(json.dumps({"impl": "reference", "unavailable": "baseline/_ref/HapHiC_cluster.py missing (run __graft_entry__.build() "
-                                                                "in the build container)"}))
+        print(json.dumps({"impl": "reference", "unavailable": REF_MISSING}))
         return
     asm = synth.make_assembly(a.nchr, a.contigs, a.mean_len, seed=a.seed)
     inflations = [float(x) for x in a.inflations.split(",")]
@@ -367,6 +433,8 @@ def run_b200(a):
     rank_id = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if world > 1:
+        if a.dump_outputs:
+            raise SystemExit("--dump-outputs: the multi-process run does not write outputs")
         from haphic_b200 import dist as hdist
         return hdist.bench_multi(a, world, rank_id, local)
 
@@ -389,8 +457,9 @@ def run_b200(a):
     def ev():
         return torch.cuda.Event(enable_timing=True)
 
-    def one_step(timed):
-        """Resident-input pass.  Returns per-stage device times (ms) and statistics."""
+    def one_step(timed, dump=None):
+        """Resident-input pass.  Returns per-stage device times (ms) and statistics.  With a `dump` dict, also copies what
+        the pass computed into it; the copying is reported as `dump_s` and left out of the stage and step times."""
         e = [ev() for _ in range(4)]
         e[0].record(stream)
         tab = LinkTable(ctx, asm.lengths, rank, in_nx, 500000, capacity_hint=hint)
@@ -404,6 +473,7 @@ def run_b200(a):
         mc = Mcl(mat)
         iters, kernel_ms, alg_bytes, products = 0, mc.normalize_ms + mc.preexp_ms, 0, mc.preexp_products
         per_infl = []
+        dump_ms, dump_s, dump_launches = 0.0, 0.0, 0
         for r in inflations:
             st = mc.run(r, a.max_iter, a.pruning)
             iters += st["rounds"]
@@ -413,10 +483,27 @@ def run_b200(a):
             per_infl.append({"inflation": r, "rounds": st["rounds"], "converged": st["converged"],
                              "ms": float(st["iter_ms"].sum()), "nnz_iter": st["iter_nnz"][:6].tolist(),
                              "ms_iter": [round(float(x), 3) for x in st["iter_ms"][:6]]})
+            if dump is not None:
+                # the next inflation overwrites this result: fetch it now, between two events the stage time leaves out
+                t0, l0, f = time.perf_counter(), ctx.launches, [ev(), ev()]
+                f[0].record(stream)
+                dump_mcl_result(dump, r, st, mc.result(), DUMP_MCL_ROWS // len(inflations))
+                f[1].record(stream)
+                f[1].synchronize()
+                dump_ms += f[0].elapsed_time(f[1])
+                dump_s += time.perf_counter() - t0
+                dump_launches += ctx.launches - l0
         e[3].record(stream)
         e[3].synchronize()
+        if dump is not None:
+            t0, l0 = time.perf_counter(), ctx.launches
+            dump_links(dump, tab, info, index, n_linked, mat, mc)
+            dump_s += time.perf_counter() - t0
+            dump_launches += ctx.launches - l0
         out = {
-            "build_ms": e[0].elapsed_time(e[1]), "matrix_ms": e[1].elapsed_time(e[2]), "mcl_ms": e[2].elapsed_time(e[3]),
+            "dump_s": dump_s, "dump_launches": dump_launches,
+            "build_ms": e[0].elapsed_time(e[1]), "matrix_ms": e[1].elapsed_time(e[2]),
+            "mcl_ms": e[2].elapsed_time(e[3]) - dump_ms,
             "iters": iters, "kernel_ms": kernel_ms, "alg_bytes": alg_bytes, "products": products,
             "nnz_full": int(info.nnz_full), "nnz_flank": int(info.nnz_flank), "n_used": int(info.n_used),
             "nnz_m0": mc.nnz_m0, "preexp_ms": mc.preexp_ms, "preexp_products": mc.preexp_products,
@@ -434,11 +521,14 @@ def run_b200(a):
     l0 = ctx.launches
     torch.cuda.synchronize()
     t_wall0 = time.perf_counter()
-    steps = [one_step(True) for _ in range(a.steps)]
+    dump = {} if a.dump_outputs else None
+    steps = [one_step(True, dump if s == a.steps - 1 else None) for s in range(a.steps)]
     torch.cuda.synchronize()
-    t_wall = time.perf_counter() - t_wall0
-    launches = ctx.launches - l0
+    t_wall = time.perf_counter() - t_wall0 - sum(s["dump_s"] for s in steps)
+    launches = ctx.launches - l0 - sum(s["dump_launches"] for s in steps)
     clocks = sampler.stop()
+    if dump is not None:
+        write_dump(a.dump_outputs, dump)
 
     if a.verbose:
         print("per-step ms:", [(round(s["build_ms"], 1), round(s["matrix_ms"], 1), round(s["mcl_ms"], 1)) for s in steps], file=sys.stderr)
@@ -531,8 +621,9 @@ def run_b200(a):
     cpu = None
     mcl_cpu = None
     if not a.no_cpu_baseline:
+        from oracle import refimpl
         cpu = cpu_baseline_block(a, asm, rank, in_nx, rec)
-        mcl_cpu = ref_mcl_small(a, inflations)
+        mcl_cpu = ref_mcl_small(a, inflations) if refimpl.available() else {"unavailable": REF_MISSING}
         # the C3 matrix itself is beyond the reference's reach (10 GB dense intermediate, hours of SpGEMM): one iteration
         # of the CPU port on a sample of columns of iterate M_1, extrapolated
         tab = LinkTable(ctx, asm.lengths, rank, in_nx, 500000, capacity_hint=hint)
