@@ -21,3 +21,5 @@ const unsigned long long* hh_links_ctg_totals(hh_links* lk);
 int32_t* hh_links_index_dev(hh_links* lk, int32_t* n_linked);
 uint8_t* hh_links_keep_dev(hh_links* lk);
 bool hh_links_finished(hh_links* lk);
+int hh_links_index_for(hh_links* lk, const uint8_t* keep, int32_t* n_linked);
+void hh_links_index_invalidate(hh_links* lk);

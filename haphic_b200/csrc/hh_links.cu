@@ -16,6 +16,7 @@
 // compaction (no sort): order[first_full] = slot, then compact.
 #include "hh_common.cuh"
 #include <stdlib.h>
+#include <algorithm>
 #include <vector>
 
 #define HH_EMPTY_KEY 0xFFFFFFFFFFFFFFFFull
@@ -91,6 +92,8 @@ struct hh_links {
     int32_t* d_index;                // [n_ctg] matrix index of linked fragments (hh_links_linked_index)
     int32_t n_linked;
     uint8_t* d_keep;
+    bool index_valid;                // d_index / n_linked / d_keep hold the result for index_keep and the current entry list
+    std::vector<uint8_t>* index_keep;
 };
 
 __device__ __forceinline__ uint64_t hh_mix64(uint64_t k) {
@@ -274,11 +277,17 @@ hh_k_links_insert(const int4* __restrict__ rec, int64_t n_rec, uint32_t stream_o
 // Partition, then aggregate.  One big hash table costs every record a random DRAM sector for the key and another
 // read-modify-write for the counters (the table is two orders of magnitude larger than L2).  For long streams the
 // records are therefore first split by the high bits of the key hash into 2^npart_log partitions (one sequential read,
-// one write in runs that fill whole sectors), and every partition is then counted in a scratch table small enough to
-// stay in L2 and emitted as compact entries (9 words, the hh_links_adopt list format).  Integer adds and mins only:
-// the result is identical to the direct path.
+// one write in runs that fill whole sectors).  A partition is still far too large for shared memory, and counting the
+// partitions one launch at a time in an L2-resident table is a chain of latency-bound launches, so every partition is
+// split again by the next hash bits into sub-partitions of at most ~1k records, and ONE launch counts all of them, a
+// CTA per sub-partition in a shared-memory table, emitting compact entries (9 words, the hh_links_adopt list format).
+// Integer adds and mins only: the result is identical to the direct path.
 //   hh_k_part_scatter   record -> {i, j, stream index, flags} (ends ordered by name rank, is_flank / head-tail evaluated once)
-//   hh_k_part_step      emit + clear the scratch table of the previous partition, count the current one into the other
+//   hh_k_sub_split      level 2: every partition (region + its spilled records) split by the next hash bits into
+//                       sub-partitions small enough for a shared-memory table (a histogram pass, then the scatter)
+//   hh_k_sub_count      one CTA per sub-partition: count in shared memory, emit the live slots
+//   hh_k_part_step      the sub-partitions whose keys did not fit the shared table: emit + clear the scratch table of the
+//                       previous one, count the current one into the other
 // ---------------------------------------------------------------------------------------------
 #define HH_PART_TILE 4096          // records per tile of the scatter kernel (512 threads x 8)
 #define HH_PART_MAX 1024
@@ -353,19 +362,270 @@ hh_k_part_scatter(const int4* __restrict__ rec, int64_t n_rec, uint32_t stream_o
     if (threadIdx.x == 0 && s_used) atomicAdd(counters + 1, (unsigned long long)s_used);
 }
 
-// count `n` partitioned records ({i, j, stream index, flags}) into a scratch table; part >= 0 selects the records of
-// that partition from a mixed list (the spill list)
-__device__ __forceinline__ void hh_part_count(const int4* __restrict__ prec, int64_t n, int part, uint64_t* __restrict__ keys,
+#define HH_SUB_MAX_LOG 10          // at most 2^10 sub-partitions per partition
+#define HH_SUB_SLOTS 2048          // slots of the shared-memory table: a sub-partition is sized for <= HH_SUB_SLOTS / 2 records
+#define HH_SUB_SMEM (HH_SUB_SLOTS * 36)   // u64 key + 7 u32 counters a slot: 72 KB, three CTAs an SM
+
+__device__ __forceinline__ unsigned hh_sub_of(const int4 r, int npart_log, int sub_log) {
+    const uint64_t key = ((uint64_t)(uint32_t)r.x << 32) | (uint64_t)(uint32_t)r.y;
+    return (unsigned)((hh_mix64(key) >> (64 - npart_log - sub_log)) & ((1ull << sub_log) - 1ull));
+}
+
+// Level 2.  blockIdx.y = the region of a partition, or (y == npart) the spill list.  !SCATTER: sub_cnt[p << sub_log | s] +=
+// records of sub-partition s of partition p.  SCATTER: record -> out[sub_off[id] + atomicAdd(sub_cnt[id])] (sub_cnt zeroed by
+// hh_k_sub_offsets), ranked inside a tile in shared memory with one global atomic per sub-partition and tile, as in
+// hh_k_part_scatter.
+template <bool SCATTER>
+__global__ void __launch_bounds__(512)
+hh_k_sub_split(const int4* __restrict__ pbuf, uint64_t pcap, const unsigned long long* __restrict__ fill, int npart_log,
+               const int4* __restrict__ spill, const unsigned long long* __restrict__ spill_fill, uint64_t spill_cap, int sub_log,
+               unsigned int* __restrict__ sub_cnt, const int64_t* __restrict__ sub_off, int4* __restrict__ out) {
+    __shared__ unsigned int s_cnt[1 << HH_SUB_MAX_LOG];
+    __shared__ unsigned long long s_base[SCATTER ? (1 << HH_SUB_MAX_LOG) : 1];
+    const int npart = 1 << npart_log, nsub = 1 << sub_log;
+    const int seg = blockIdx.y;
+    if (seg == npart) {
+        // the spill list (skewed streams only): records of any partition, which they carry in their flags
+        const int64_t n = (int64_t)min(*spill_fill, (unsigned long long)spill_cap);
+        for (int64_t i = (int64_t)blockIdx.x * 512 + threadIdx.x; i < n; i += (int64_t)gridDim.x * 512) {
+            const int4 r = spill[i];
+            const unsigned id = (((unsigned)r.w >> 8) << sub_log) | hh_sub_of(r, npart_log, sub_log);
+            if (SCATTER) out[sub_off[id] + atomicAdd(sub_cnt + id, 1u)] = r;
+            else atomicAdd(sub_cnt + id, 1u);
+        }
+        return;
+    }
+    const int4* src = pbuf + (size_t)seg * (size_t)pcap;
+    const int64_t n = (int64_t)min(fill[seg], (unsigned long long)pcap);      // the excess is on the spill list
+    unsigned int* cnt = sub_cnt + ((size_t)seg << sub_log);
+    const int64_t tiles = (n + HH_PART_TILE - 1) / HH_PART_TILE;
+    for (int k = threadIdx.x; k < nsub; k += 512) s_cnt[k] = 0;
+    __syncthreads();
+    for (int64_t t = blockIdx.x; t < tiles; t += gridDim.x) {
+        int4 r[8];
+        int s[8];
+        unsigned int rnk[8];
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+            const int64_t i = t * HH_PART_TILE + (int64_t)k * 512 + threadIdx.x;
+            s[k] = -1;
+            if (i < n) {
+                r[k] = hh_ld_stream(src + i);
+                s[k] = (int)hh_sub_of(r[k], npart_log, sub_log);
+                if (SCATTER) rnk[k] = atomicAdd(&s_cnt[s[k]], 1u);
+                else atomicAdd(&s_cnt[s[k]], 1u);
+            }
+        }
+        if (SCATTER) {
+            __syncthreads();
+            for (int k = threadIdx.x; k < nsub; k += 512)
+                if (s_cnt[k]) s_base[k] = (unsigned long long)sub_off[((size_t)seg << sub_log) + k] + atomicAdd(cnt + k, s_cnt[k]);
+            __syncthreads();
+#pragma unroll
+            for (int k = 0; k < 8; ++k)
+                if (s[k] >= 0) out[s_base[s[k]] + rnk[k]] = r[k];
+            __syncthreads();
+            for (int k = threadIdx.x; k < nsub; k += 512) s_cnt[k] = 0;
+            __syncthreads();
+        }
+    }
+    if (!SCATTER) {
+        __syncthreads();
+        for (int k = threadIdx.x; k < nsub; k += 512)
+            if (s_cnt[k]) atomicAdd(cnt + k, s_cnt[k]);
+    }
+}
+
+// sub_off[p << sub_log | s] = pbase[p] + records of sub-partitions 0 .. s-1 of partition p (one CTA a partition); sub_cnt is
+// cleared for the scatter.  pbase = exclusive prefix of the partition totals, which the host has from the level-1 cursors.
+__global__ void __launch_bounds__(1024)
+hh_k_sub_offsets(unsigned int* __restrict__ sub_cnt, int sub_log, const int64_t* __restrict__ pbase, int npart,
+                 int64_t* __restrict__ sub_off) {
+    __shared__ unsigned int s_w[32];
+    const int nsub = 1 << sub_log, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const size_t at = ((size_t)blockIdx.x << sub_log) + threadIdx.x;
+    const unsigned int v = (int)threadIdx.x < nsub ? sub_cnt[at] : 0u;
+    unsigned int incl = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const unsigned int t = __shfl_up_sync(HH_FULL_MASK, incl, o);
+        if (lane >= o) incl += t;
+    }
+    if (lane == 31) s_w[warp] = incl;
+    __syncthreads();
+    if (warp == 0) {
+        const unsigned int w = s_w[lane];
+        unsigned int wi = w;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned int t = __shfl_up_sync(HH_FULL_MASK, wi, o);
+            if (lane >= o) wi += t;
+        }
+        s_w[lane] = wi - w;
+    }
+    __syncthreads();
+    if ((int)threadIdx.x < nsub) {
+        sub_off[at] = pbase[blockIdx.x] + (int64_t)(s_w[warp] + incl - v);
+        sub_cnt[at] = 0u;
+    }
+    if (blockIdx.x == npart - 1 && threadIdx.x == 0) sub_off[(size_t)npart << sub_log] = pbase[npart];
+}
+
+// Count + emit: a CTA takes sub-partitions in a grid stride, counts each into an open-addressing table in shared memory
+// (warp aggregation with match.any as in hh_part_count, then shared-memory atomics), and emits the live slots with a block
+// scan and ONE global atomic on the entry cursor.  Nothing global is touched before the emit.  A sub-partition whose keys do
+// not fit the table (skewed or adversarial keys only) is abandoned and its id appended to `fallback` (counters[7] entries)
+// for the global scratch-table path (hh_k_part_step).
+__global__ void __launch_bounds__(256)
+hh_k_sub_count(const int4* __restrict__ prec, const int64_t* __restrict__ sub_off, int nsub_total, uint32_t* __restrict__ compact,
+               uint64_t compact_cap, unsigned long long* __restrict__ ctg_links, unsigned long long* __restrict__ counters,
+               uint32_t* __restrict__ fallback) {
+    constexpr int S = HH_SUB_SLOTS, E = HH_SUB_SLOTS / 256;
+    extern __shared__ uint64_t s_keys[];                   // [S], then 7 x u32 [S]
+    uint32_t* s_ff = reinterpret_cast<uint32_t*>(s_keys + S);
+    uint32_t* s_ffl = s_ff + S;
+    uint32_t* s_full = s_ffl + S;
+    uint32_t* s_fl = s_full + S;
+    uint32_t* s_ht = s_fl + S;
+    uint32_t* s_th = s_ht + S;
+    uint32_t* s_tt = s_th + S;
+    __shared__ unsigned int s_over, s_wtot[8];
+    __shared__ unsigned long long s_base;
+    const int lane = threadIdx.x & 31, wv = threadIdx.x >> 5;
+    unsigned int nfl = 0;
+    for (int id = blockIdx.x; id < nsub_total; id += gridDim.x) {
+        for (int k = threadIdx.x; k < S; k += 256) {
+            s_keys[k] = HH_EMPTY_KEY;
+            s_ff[k] = HH_NONE32;
+            s_ffl[k] = HH_NONE32;
+            s_full[k] = 0u;
+            s_fl[k] = 0u;
+            s_ht[k] = 0u;
+            s_th[k] = 0u;
+            s_tt[k] = 0u;
+        }
+        if (threadIdx.x == 0) s_over = 0u;
+        __syncthreads();
+        const int64_t b = sub_off[id], n = sub_off[id + 1] - b;
+        for (int64_t i0 = (int64_t)wv * 32; i0 < n; i0 += 256) {
+            if (__any_sync(HH_FULL_MASK, *(volatile unsigned int*)&s_over != 0u)) break;
+            const int64_t i = i0 + lane;
+            const bool ok = i < n;
+            int4 r = make_int4(0, 0, 0, 0);
+            if (ok) r = hh_ld_stream(prec + b + i);
+            const unsigned f = (unsigned)r.w;
+            const uint64_t key = ok ? (((uint64_t)(uint32_t)r.x << 32) | (uint64_t)(uint32_t)r.y) : (HH_EMPTY_KEY - 1 - (uint64_t)lane);
+            const unsigned peers = __match_any_sync(HH_FULL_MASK, key);
+            const bool fl = ok && (f & 1u), ti = (f & 2u) != 0, tj = (f & 4u) != 0;
+            const uint32_t idx = ok ? (uint32_t)r.z : HH_NONE32;
+            const uint32_t first_all = __reduce_min_sync(peers, idx);
+            const uint32_t first_fl = __reduce_min_sync(peers, fl ? idx : HH_NONE32);
+            const unsigned b_fl = __ballot_sync(HH_FULL_MASK, fl);
+            const unsigned b_ht = __ballot_sync(HH_FULL_MASK, ok && !ti && tj);
+            const unsigned b_th = __ballot_sync(HH_FULL_MASK, ok && ti && !tj);
+            const unsigned b_tt = __ballot_sync(HH_FULL_MASK, ok && ti && tj);
+            if (ok && lane == (__ffs(peers) - 1)) {
+                unsigned int sl = (unsigned int)hh_mix64(key) & (S - 1);     // the low hash bits; the partition ids took the high ones
+                bool found = false;
+                for (int q = 0; q < S; ++q) {
+                    const uint64_t k = *((volatile uint64_t*)(s_keys + sl));
+                    if (k == key) { found = true; break; }
+                    if (k == HH_EMPTY_KEY) {
+                        const unsigned long long prev = atomicCAS((unsigned long long*)(s_keys + sl), (unsigned long long)HH_EMPTY_KEY,
+                                                                  (unsigned long long)key);
+                        if (prev == HH_EMPTY_KEY || prev == key) { found = true; break; }
+                    }
+                    sl = (sl + 1) & (S - 1);
+                }
+                if (!found) {
+                    s_over = 1u;
+                } else {
+                    const unsigned c_fl = __popc(peers & b_fl), c_ht = __popc(peers & b_ht), c_th = __popc(peers & b_th),
+                                   c_tt = __popc(peers & b_tt);
+                    atomicAdd(s_full + sl, (unsigned)__popc(peers));
+                    atomicMin(s_ff + sl, first_all);
+                    if (c_fl) {
+                        atomicAdd(s_fl + sl, c_fl);
+                        atomicMin(s_ffl + sl, first_fl);
+                    }
+                    if (c_ht) atomicAdd(s_ht + sl, c_ht);
+                    if (c_th) atomicAdd(s_th + sl, c_th);
+                    if (c_tt) atomicAdd(s_tt + sl, c_tt);
+                }
+            }
+        }
+        __syncthreads();
+        if (s_over) {
+            if (threadIdx.x == 0) fallback[atomicAdd(counters + 7, 1ull)] = (uint32_t)id;
+            __syncthreads();                   // s_over is read by every thread before the next sub-partition resets it
+            continue;
+        }
+        // ---- emit: live slots -> compact entries {i, j, full, flank, first_full, first_flank, HT, TH, TT}, per-fragment totals
+        unsigned int cnt = 0;
+#pragma unroll
+        for (int q = 0; q < E; ++q) cnt += (s_keys[q * 256 + threadIdx.x] != HH_EMPTY_KEY) ? 1u : 0u;
+        unsigned int incl = cnt;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned int t = __shfl_up_sync(HH_FULL_MASK, incl, o);
+            if (lane >= o) incl += t;
+        }
+        if (lane == 31) s_wtot[wv] = incl;
+        __syncthreads();
+        unsigned int before = 0, total = 0;
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+            const unsigned int t = s_wtot[k];
+            before += (k < wv) ? t : 0u;
+            total += t;
+        }
+        if (threadIdx.x == 0) s_base = total ? atomicAdd(counters + 0, (unsigned long long)total) : 0ull;
+        __syncthreads();
+        unsigned long long pos = s_base + before + (incl - cnt);
+#pragma unroll
+        for (int q = 0; q < E; ++q) {
+            const int sl = q * 256 + threadIdx.x;
+            const uint64_t key = s_keys[sl];
+            if (key == HH_EMPTY_KEY) continue;
+            const uint32_t flank = s_fl[sl];
+            if (pos < compact_cap) {
+                uint32_t* o = compact + pos * 9;
+                o[0] = (uint32_t)(key >> 32);
+                o[1] = (uint32_t)key;
+                o[2] = s_full[sl];
+                o[3] = flank;
+                o[4] = s_ff[sl];
+                o[5] = s_ffl[sl];
+                o[6] = s_ht[sl];
+                o[7] = s_th[sl];
+                o[8] = s_tt[sl];
+            } else {
+                atomicExch(counters + 2, 5ull);
+            }
+            pos++;
+            if (flank) {
+                nfl++;
+                atomicAdd(ctg_links + (uint32_t)(key >> 32), (unsigned long long)flank);      // ctg_link_dict (1638-1639)
+                atomicAdd(ctg_links + (uint32_t)key, (unsigned long long)flank);
+            }
+        }
+        __syncthreads();                       // the table and s_wtot / s_base are reused by the next sub-partition
+    }
+    nfl = (unsigned)hh_warp_sum((int)nfl);
+    if (lane == 0 && nfl) atomicAdd(counters + 3, (unsigned long long)nfl);
+}
+
+// count `n` partitioned records ({i, j, stream index, flags}) into a scratch table
+__device__ __forceinline__ void hh_part_count(const int4* __restrict__ prec, int64_t n, uint64_t* __restrict__ keys,
                                               hh_slot* __restrict__ vals, uint64_t cap, unsigned long long* __restrict__ counters) {
     const int lane = threadIdx.x & 31;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i0 = (int64_t)blockIdx.x * blockDim.x + (threadIdx.x - lane); i0 < n; i0 += stride) {
         const int64_t i = i0 + lane;
-        bool ok = i < n;
+        const bool ok = i < n;
         int4 r = make_int4(0, 0, 0, 0);
         if (ok) r = hh_ld_stream(prec + i);
         const unsigned f = (unsigned)r.w;
-        if (ok && part >= 0) ok = (int)(f >> 8) == part;
         const uint64_t key = ok ? (((uint64_t)(uint32_t)r.x << 32) | (uint64_t)(uint32_t)r.y) : (HH_EMPTY_KEY - 1 - (uint64_t)lane);
         const unsigned peers = __match_any_sync(HH_FULL_MASK, key);
         const bool fl = ok && (f & 1u), ti = (f & 2u) != 0, tj = (f & 4u) != 0;
@@ -391,8 +651,7 @@ __device__ __forceinline__ void hh_part_count(const int4* __restrict__ prec, int
 }
 
 __global__ void __launch_bounds__(256)
-hh_k_part_step(const int4* __restrict__ prec, int64_t n, const int4* __restrict__ spill, int64_t n_spill, int part,
-               uint64_t* __restrict__ ckeys, hh_slot* __restrict__ cvals, uint64_t* __restrict__ ekeys, hh_slot* __restrict__ evals, uint64_t cap,
+hh_k_part_step(const int4* __restrict__ prec, int64_t n, uint64_t* __restrict__ ckeys, hh_slot* __restrict__ cvals, uint64_t* __restrict__ ekeys, hh_slot* __restrict__ evals, uint64_t cap,
                uint32_t* __restrict__ compact, uint64_t compact_cap, unsigned long long* __restrict__ ctg_links,
                unsigned long long* __restrict__ counters) {
     // ---- emit the table of the previous partition: live slots -> compact entries, per-fragment totals; slots are cleared.
@@ -477,11 +736,8 @@ hh_k_part_step(const int4* __restrict__ prec, int64_t n, const int4* __restrict_
         nfl = (unsigned)hh_warp_sum((int)nfl);
         if (lane == 0 && nfl) atomicAdd(counters + 3, (unsigned long long)nfl);
     }
-    // ---- count the current partition
-    if (ckeys != nullptr) {
-        if (n > 0) hh_part_count(prec, n, -1, ckeys, cvals, cap, counters);
-        if (n_spill > 0) hh_part_count(spill, n_spill, part, ckeys, cvals, cap, counters);
-    }
+    // ---- count the current sub-partition
+    if (ckeys != nullptr && n > 0) hh_part_count(prec, n, ckeys, cvals, cap, counters);
 }
 
 // re-insert every live slot of the old table into a (larger) new one
@@ -749,26 +1005,73 @@ __global__ void hh_k_touch(const uint32_t* __restrict__ compact, int64_t nnz, co
     }
 }
 
-// index[c] = number of touched fragments touched earlier than c (touch values are unique)
-__global__ void __launch_bounds__(256)
-hh_k_rank_touch(const unsigned long long* __restrict__ touch, int n, int32_t* __restrict__ index, int* __restrict__ n_linked) {
-    __shared__ unsigned long long tile[1024];
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    const unsigned long long mine = (c < n) ? touch[c] : ~0ull;
-    int rank = 0;
-    for (int base = 0; base < n; base += 1024) {
-        for (int k = threadIdx.x; k < 1024; k += blockDim.x) tile[k] = (base + k < n) ? touch[base + k] : ~0ull;
-        __syncthreads();
-        if (mine != ~0ull) {
-#pragma unroll 8
-            for (int k = 0; k < 1024; ++k) rank += (tile[k] < mine) ? 1 : 0;
-        }
-        __syncthreads();
-    }
+// index[c] = number of touched fragments touched earlier than c (touch values are unique): the position of c in a sort of
+// the (touch, fragment) pairs.  Untouched fragments (touch ~0) sort after every touched one.  A stable LSD radix sort,
+// 8-bit digits, tiles of 1024 pairs (one per thread): touch < 2^33, so five passes over bits 0..39 order it.
+#define HH_RADIX_TILE 1024
+#define HH_RADIX_PASSES 5
+
+__global__ void __launch_bounds__(HH_RADIX_TILE)
+hh_k_rank_init(const unsigned long long* __restrict__ touch, int n, unsigned long long* __restrict__ key, int32_t* __restrict__ val,
+               int* __restrict__ n_linked) {
+    const int c = blockIdx.x * HH_RADIX_TILE + threadIdx.x;
+    int touched = 0;
     if (c < n) {
-        index[c] = (mine != ~0ull) ? rank : -1;
-        if (mine != ~0ull) atomicAdd(n_linked, 1);
+        key[c] = touch[c];
+        val[c] = c;
+        touched = touch[c] != ~0ull;
     }
+    touched = hh_warp_sum(touched);
+    if ((threadIdx.x & 31) == 0 && touched) atomicAdd(n_linked, touched);
+}
+
+// cnt[digit * n_tiles + tile] = pairs of the tile with that digit
+__global__ void __launch_bounds__(HH_RADIX_TILE)
+hh_k_radix_hist(const unsigned long long* __restrict__ key, int n, int shift, int* __restrict__ cnt) {
+    __shared__ int s_h[256];
+    if (threadIdx.x < 256) s_h[threadIdx.x] = 0;
+    __syncthreads();
+    const int i = blockIdx.x * HH_RADIX_TILE + threadIdx.x;
+    if (i < n) atomicAdd(&s_h[(key[i] >> shift) & 255u], 1);
+    __syncthreads();
+    if (threadIdx.x < 256) cnt[(size_t)threadIdx.x * gridDim.x + blockIdx.x] = s_h[threadIdx.x];
+}
+
+// stable scatter: off = exclusive scan of cnt; inside the tile, the rank among equal digits of the lower warps and lanes
+__global__ void __launch_bounds__(HH_RADIX_TILE)
+hh_k_radix_scatter(const unsigned long long* __restrict__ key, const int32_t* __restrict__ val, int n, int shift,
+                   const int64_t* __restrict__ off, unsigned long long* __restrict__ key_out, int32_t* __restrict__ val_out) {
+    __shared__ int s_w[32][256];               // digit counts of every warp, then their exclusive prefix over the warps
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int k = threadIdx.x; k < 32 * 256; k += HH_RADIX_TILE) s_w[k >> 8][k & 255] = 0;
+    __syncthreads();
+    const int i = blockIdx.x * HH_RADIX_TILE + threadIdx.x;
+    const bool ok = i < n;
+    const unsigned long long k = ok ? key[i] : 0ull;
+    const int d = ok ? (int)((k >> shift) & 255u) : -1;
+    const unsigned peers = __match_any_sync(HH_FULL_MASK, d);
+    const int rank = __popc(peers & ((1u << lane) - 1u));
+    if (ok && rank == 0) s_w[warp][d] = __popc(peers);
+    __syncthreads();
+    if (threadIdx.x < 256) {
+        int run = 0;
+        for (int w = 0; w < 32; ++w) {
+            const int t = s_w[w][threadIdx.x];
+            s_w[w][threadIdx.x] = run;
+            run += t;
+        }
+    }
+    __syncthreads();
+    if (ok) {
+        const int64_t q = off[(size_t)d * gridDim.x + blockIdx.x] + s_w[warp][d] + rank;
+        key_out[q] = k;
+        val_out[q] = val[i];
+    }
+}
+
+__global__ void hh_k_rank_index(const int32_t* __restrict__ val, int n, const int* __restrict__ n_linked, int32_t* __restrict__ index) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r < n) index[val[r]] = (r < *n_linked) ? r : -1;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -884,6 +1187,7 @@ static int links_create_common(hh_ctx* ctx, int32_t n_key, const int64_t* key_le
     HH_CUDA(cudaStreamSynchronize(st));   // host temporaries go out of scope
     lk->capacity_hint = capacity_hint;
     lk->psets = new std::vector<hh_partset>();
+    lk->index_keep = new std::vector<uint8_t>();
     HH_CUDA(cudaStreamCreateWithFlags(&lk->copy_stream, cudaStreamNonBlocking));
     for (int k = 0; k < 2; ++k) {
         HH_CUDA(cudaEventCreateWithFlags(&lk->ev_copied[k], cudaEventDisableTiming));
@@ -1069,8 +1373,7 @@ extern "C" int hh_links_add(hh_links* lk, const int32_t* rec, int64_t n_rec, int
     return HH_OK;
 }
 
-// partitioned counting, second phase: every partition through an L2-resident scratch table (two tables, so the emit of
-// partition p - 1 and the count of partition p share one launch), entries appended to an unordered compact list
+// partitioned counting, second phase: level-2 split, shared-memory count + emit, and the scratch-table fallback
 static void links_free_partsets(hh_links* lk) {
     if (lk->psets) {
         for (size_t k = 0; k < lk->psets->size(); ++k) {
@@ -1087,65 +1390,115 @@ static int links_finish_partitioned(hh_links* lk) {
     hh_ctx* ctx = lk->ctx;
     const int npart = 1 << lk->npart_log;
     const size_t nsets = lk->psets->size();
+    // one read-back: the counters, the level-1 region fill levels and the spill count
+    std::vector<unsigned long long> fill(nsets * (size_t)npart);
+    unsigned long long n_spill = 0;
+    HH_CUDA(cudaMemcpyAsync(ctx->h_scratch, lk->d_counters, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+    for (size_t k = 0; k < nsets; ++k)
+        HH_CUDA(cudaMemcpyAsync(fill.data() + k * (size_t)npart, (*lk->psets)[k].cursor, (size_t)npart * sizeof(unsigned long long),
+                                cudaMemcpyDeviceToHost, ctx->stream));
+    HH_CUDA(cudaMemcpyAsync(&n_spill, lk->d_spill_cursor, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+    HH_CUDA(cudaStreamSynchronize(ctx->stream));
     unsigned long long c[8];
-    HH_CHECK(links_read_counters(lk, c));
+    for (int k = 0; k < 8; ++k) c[k] = ctx->h_scratch[k];
     HH_REQUIRE(c[2] == 0, HH_ERR_CAPACITY,
                "hh_links_finish: the spill list of the partitioned counting overflowed (a few contig pairs own most of the stream): "
                "set HH_LINKS_PARTITION=0 to use the direct hash table");
     lk->n_used = lk->peer_used + (int64_t)c[1];
-    // region fill levels and the spill count
-    std::vector<unsigned long long> fill(nsets * (size_t)npart);
-    for (size_t k = 0; k < nsets; ++k)
-        HH_CUDA(cudaMemcpyAsync(fill.data() + k * (size_t)npart, (*lk->psets)[k].cursor, (size_t)npart * sizeof(unsigned long long),
-                                cudaMemcpyDeviceToHost, ctx->stream));
-    unsigned long long n_spill = 0;
-    HH_CUDA(cudaMemcpyAsync(&n_spill, lk->d_spill_cursor, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
-    HH_CUDA(cudaStreamSynchronize(ctx->stream));
-    // scratch tables: load factor <= 0.6 even if every record of the fullest partition is a distinct key
-    unsigned long long worst = 1;
+    // partition totals (a cursor counts every record of its partition, the spilled ones included), their exclusive prefix
+    // (where each partition starts in the level-2 buffer), and the level-2 fan-out: the fullest partition split into
+    // sub-partitions of at most HH_SUB_SLOTS / 2 records, so that even all-distinct keys fill the shared table at most half
+    std::vector<int64_t> pbase((size_t)npart + 1, 0);
+    int64_t worst = 1, region = (int64_t)n_spill;
     for (int p = 0; p < npart; ++p) {
-        unsigned long long t = 0;
-        for (size_t k = 0; k < nsets; ++k) t += fill[k * (size_t)npart + p];
-        if (t > worst) worst = t;
+        int64_t t = 0;
+        for (size_t k = 0; k < nsets; ++k) {
+            const unsigned long long f = fill[k * (size_t)npart + p];
+            t += (int64_t)f;
+            region = std::max(region, (int64_t)std::min(f, (unsigned long long)(*lk->psets)[k].pcap));
+        }
+        pbase[p + 1] = pbase[p] + t;
+        worst = std::max(worst, t);
     }
-    uint64_t scap = 1ull << 12;
-    while ((double)scap * 0.6 < (double)worst) scap <<= 1;
-    lk->scap = scap;
-    uint64_t* skeys[2] = {nullptr, nullptr};
-    hh_slot* svals[2] = {nullptr, nullptr};
+    const int sub_max = std::min(HH_SUB_MAX_LOG, std::max(0, links_env_int("HH_LINKS_SUB_LOG_MAX", HH_SUB_MAX_LOG)));
+    int sub_log = 0;
+    while (sub_log < sub_max && (worst >> sub_log) > HH_SUB_SLOTS / 2) sub_log++;
+    const int nsub = npart << sub_log;
+    const int64_t total = pbase[npart];
     const uint64_t compact_cap = (uint64_t)(lk->n_used > 0 ? lk->n_used : 1);       // distinct pairs <= usable records
     hh_dfree(lk->d_compact);
-    uint32_t* d_stage_compact = nullptr;                                              // workspace; the exact-size list is cut from it
+    int4* d_rec2 = nullptr;                       // level-2 buffer: sub-partition id after sub-partition id
+    uint32_t* d_stage_compact = nullptr;          // workspace; the exact-size list is cut from it
+    unsigned int* d_cnt = nullptr;
+    int64_t* d_off = nullptr;
+    int64_t* d_pbase = nullptr;
+    uint32_t* d_fb = nullptr;
+    uint64_t* skeys[2] = {nullptr, nullptr};
+    hh_slot* svals[2] = {nullptr, nullptr};
     int rc = [&]() -> int {
+        HH_CHECK(hh_ws_alloc(ctx, &d_rec2, (size_t)(total > 0 ? total : 1)));
         HH_CHECK(hh_ws_alloc(ctx, &d_stage_compact, (size_t)compact_cap * 9));
-        for (int b = 0; b < 2; ++b) HH_CHECK(links_alloc_table(lk, scap, &skeys[b], &svals[b]));
+        HH_CHECK(hh_dmalloc(&d_cnt, (size_t)nsub));
+        HH_CHECK(hh_dmalloc(&d_off, (size_t)nsub + 1));
+        HH_CHECK(hh_dmalloc(&d_pbase, (size_t)npart + 1));
+        HH_CHECK(hh_dmalloc(&d_fb, (size_t)nsub));
+        HH_CUDA(cudaMemsetAsync(d_cnt, 0, (size_t)nsub * sizeof(unsigned int), ctx->stream));
+        HH_CUDA(cudaMemcpyAsync(d_pbase, pbase.data(), ((size_t)npart + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
         HH_CUDA(cudaMemsetAsync(lk->d_counters + 0, 0, sizeof(unsigned long long), ctx->stream));     // entry cursor
         HH_CUDA(cudaMemsetAsync(lk->d_counters + 3, 0, sizeof(unsigned long long), ctx->stream));     // nnz_flank
-        const int grid = hh_grid(ctx, 8);
-        for (int p = 0; p <= npart; ++p) {
-            const int cb = p & 1, eb = cb ^ 1;
-            bool first = true;
-            for (size_t k = 0; k < nsets || first; ++k) {
-                const bool have = p < npart && k < nsets;
-                const uint64_t pcap = k < nsets ? (*lk->psets)[k].pcap : 0;
-                unsigned long long nrec = have ? fill[k * (size_t)npart + p] : 0;
-                if (have && nrec > pcap) nrec = pcap;                 // the excess is on the spill list
-                const int4* prec = have ? (*lk->psets)[k].buf + (size_t)p * (size_t)pcap : nullptr;
-                // the spill list is scanned once per overflowed partition (with the first set)
-                bool spill_now = false;
-                if (p < npart && first && n_spill) {
-                    for (size_t kk = 0; kk < nsets; ++kk) spill_now = spill_now || fill[kk * (size_t)npart + p] > (*lk->psets)[kk].pcap;
-                }
-                HH_LAUNCH(ctx, hh_k_part_step, grid, 256, 0, prec, (int64_t)nrec, lk->d_spill, spill_now ? (int64_t)n_spill : 0, p,
-                          p < npart ? skeys[cb] : nullptr, p < npart ? svals[cb] : nullptr, (first && p > 0) ? skeys[eb] : nullptr,
-                          (first && p > 0) ? svals[eb] : nullptr, scap, d_stage_compact, compact_cap, lk->d_ctg, lk->d_counters);
-                first = false;
-                if (k + 1 >= nsets) break;
+        HH_CUDA(cudaMemsetAsync(lk->d_counters + 7, 0, sizeof(unsigned long long), ctx->stream));     // fallback sub-partitions
+        // level 2: histogram, offsets, scatter (the spill list goes with the first set)
+        const int gx = (int)std::min<int64_t>(64, (region + HH_PART_TILE - 1) / HH_PART_TILE + 1);
+        for (int pass = 0; pass < 2; ++pass) {
+            if (pass == 1) HH_LAUNCH(ctx, hh_k_sub_offsets, npart, 1024, 0, d_cnt, sub_log, d_pbase, npart, d_off);
+            for (size_t k = 0; k < nsets; ++k) {
+                const hh_partset& ps = (*lk->psets)[k];
+                const dim3 grid(gx, npart + (k == 0 ? 1 : 0));
+                if (pass == 0)
+                    HH_LAUNCH(ctx, hh_k_sub_split<false>, grid, 512, 0, ps.buf, ps.pcap, ps.cursor, lk->npart_log, lk->d_spill,
+                              lk->d_spill_cursor, lk->spill_cap, sub_log, d_cnt, (const int64_t*)nullptr, (int4*)nullptr);
+                else
+                    HH_LAUNCH(ctx, hh_k_sub_split<true>, grid, 512, 0, ps.buf, ps.pcap, ps.cursor, lk->npart_log, lk->d_spill,
+                              lk->d_spill_cursor, lk->spill_cap, sub_log, d_cnt, d_off, d_rec2);
             }
         }
+        // count + emit in shared memory
+        HH_CUDA(cudaFuncSetAttribute(hh_k_sub_count, cudaFuncAttributeMaxDynamicSharedMemorySize, HH_SUB_SMEM));
+        int per_sm = 0;
+        HH_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, hh_k_sub_count, 256, HH_SUB_SMEM));
+        const int grid = (int)std::min<int64_t>(nsub, (int64_t)ctx->sm_count * std::max(per_sm, 1));
+        HH_LAUNCH(ctx, hh_k_sub_count, grid, 256, HH_SUB_SMEM, d_rec2, d_off, nsub, d_stage_compact, compact_cap, lk->d_ctg,
+                  lk->d_counters, d_fb);
         HH_CHECK(links_read_counters(lk, c));
+        lk->scap = HH_SUB_SLOTS;
+        if (c[7] && c[2] == 0) {
+            // sub-partitions whose keys did not fit the shared table, one after the other through a global scratch table
+            // (two tables, so the emit of one and the count of the next share a launch)
+            const size_t nfb = (size_t)c[7];
+            std::vector<uint32_t> fb(nfb);
+            std::vector<int64_t> off((size_t)nsub + 1);
+            HH_CUDA(cudaMemcpyAsync(fb.data(), d_fb, nfb * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+            HH_CUDA(cudaMemcpyAsync(off.data(), d_off, ((size_t)nsub + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+            HH_CUDA(cudaStreamSynchronize(ctx->stream));
+            int64_t big = 1;
+            for (size_t f = 0; f < nfb; ++f) big = std::max(big, off[fb[f] + 1] - off[fb[f]]);
+            uint64_t scap = 1ull << 12;
+            while ((double)scap * 0.6 < (double)big) scap <<= 1;          // load factor <= 0.6 even for all-distinct keys
+            lk->scap = scap;
+            for (int b = 0; b < 2; ++b) HH_CHECK(links_alloc_table(lk, scap, &skeys[b], &svals[b]));
+            const int grid2 = hh_grid(ctx, 8);
+            for (size_t f = 0; f <= nfb; ++f) {
+                const int cb = (int)(f & 1), eb = cb ^ 1;
+                const bool cur = f < nfb;
+                const int64_t b0 = cur ? off[fb[f]] : 0, n = cur ? off[fb[f] + 1] - b0 : 0;
+                HH_LAUNCH(ctx, hh_k_part_step, grid2, 256, 0, cur ? d_rec2 + b0 : nullptr, n, cur ? skeys[cb] : nullptr,
+                          cur ? svals[cb] : nullptr, f > 0 ? skeys[eb] : nullptr, f > 0 ? svals[eb] : nullptr, scap, d_stage_compact,
+                          compact_cap, lk->d_ctg, lk->d_counters);
+            }
+            HH_CHECK(links_read_counters(lk, c));
+        }
         HH_REQUIRE(c[2] == 0, HH_ERR_CAPACITY,
-                   "hh_links_finish: a scratch table of the partitioned counting overflowed (code %llu): set HH_LINKS_PARTITION=0", c[2]);
+                   "hh_links_finish: a table of the partitioned counting overflowed (code %llu): set HH_LINKS_PARTITION=0", c[2]);
         lk->nnz = (int64_t)c[0];
         lk->nnz_flank = (int64_t)c[3];
         HH_CHECK(hh_dmalloc(&lk->d_compact, (size_t)(lk->nnz > 0 ? lk->nnz : 1) * 9));
@@ -1154,7 +1507,12 @@ static int links_finish_partitioned(hh_links* lk) {
                                     ctx->stream));
         return HH_OK;
     }();
+    hh_ws_free(ctx, d_rec2);
     hh_ws_free(ctx, d_stage_compact);
+    hh_dfree(d_cnt);
+    hh_dfree(d_off);
+    hh_dfree(d_pbase);
+    hh_dfree(d_fb);
     for (int b = 0; b < 2; ++b) {
         hh_dfree(skeys[b]);
         hh_dfree(svals[b]);
@@ -1163,6 +1521,7 @@ static int links_finish_partitioned(hh_links* lk) {
     HH_CHECK(rc);
     lk->finished = true;
     lk->ordered = false;        // dict insertion order is restored by the first hh_links_fetch (links_order_list)
+    lk->index_valid = false;
     return HH_OK;
 }
 
@@ -1222,6 +1581,7 @@ extern "C" int hh_links_finish(hh_links* lk, hh_links_info* info) {
         }
         lk->finished = true;
         lk->ordered = true;
+        lk->index_valid = false;
     }
     if (info) {
         info->n_records = lk->n_records;
@@ -1375,6 +1735,7 @@ extern "C" int hh_links_finish_partition(hh_links* lk, hh_links_info* info) {
         }
         lk->finished = true;
         lk->ordered = false;
+        lk->index_valid = false;
     }
     if (info) {
         info->n_records = lk->n_records;
@@ -1423,6 +1784,7 @@ extern "C" int hh_links_adopt(hh_links* lk, const uint32_t* entries_dev, int64_t
     lk->stream_end = stream_end;
     lk->finished = true;
     lk->ordered = false;
+    lk->index_valid = false;
     return HH_OK;
 }
 
@@ -1539,6 +1901,7 @@ extern "C" int hh_links_merge(hh_links* lk, const uint32_t* entries_dev, int64_t
     lk->mode = 1;
     HH_CHECK(links_need_table(lk));
     lk->finished = false;   // a finished table is re-opened: the next hh_links_finish rebuilds the ordered view
+    lk->index_valid = false;
     HH_REQUIRE(n_entries >= 0 && (entries_dev || n_entries == 0), HH_ERR_ARG, "hh_links_merge: bad entries");
     hh_ctx* ctx = lk->ctx;
     HH_CUDA(cudaSetDevice(ctx->device));
@@ -1563,11 +1926,24 @@ extern "C" int hh_links_linked_index(hh_links* lk, const uint8_t* keep, int32_t*
     HH_REQUIRE(lk->finished, HH_ERR_STATE, "hh_links_linked_index: call hh_links_finish first");
     hh_ctx* ctx = lk->ctx;
     HH_CUDA(cudaSetDevice(ctx->device));
+    lk->index_valid = false;
+    const int n = lk->n_ctg;
+    const int nb = (n + HH_RADIX_TILE - 1) / HH_RADIX_TILE;
     unsigned long long* d_touch = nullptr;
-    HH_CHECK(hh_dmalloc(&d_touch, (size_t)lk->n_ctg));
+    unsigned long long* d_key[2] = {nullptr, nullptr};
+    int32_t* d_val[2] = {nullptr, nullptr};
+    int* d_cnt = nullptr;
+    int64_t* d_off = nullptr;
     int rc = [&]() -> int {
-        HH_CUDA(cudaMemcpyAsync(lk->d_keep, keep, (size_t)lk->n_ctg, cudaMemcpyHostToDevice, ctx->stream));
-        HH_CUDA(cudaMemsetAsync(d_touch, 0xFF, (size_t)lk->n_ctg * sizeof(unsigned long long), ctx->stream));
+        HH_CHECK(hh_dmalloc(&d_touch, (size_t)n));
+        for (int b = 0; b < 2; ++b) {
+            HH_CHECK(hh_dmalloc(&d_key[b], (size_t)n));
+            HH_CHECK(hh_dmalloc(&d_val[b], (size_t)n));
+        }
+        HH_CHECK(hh_dmalloc(&d_cnt, (size_t)nb * 256));
+        HH_CHECK(hh_dmalloc(&d_off, (size_t)nb * 256 + 1));
+        HH_CUDA(cudaMemcpyAsync(lk->d_keep, keep, (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+        HH_CUDA(cudaMemsetAsync(d_touch, 0xFF, (size_t)n * sizeof(unsigned long long), ctx->stream));
         int* d_nl = reinterpret_cast<int*>(ctx->d_scratch + 8);
         HH_CUDA(cudaMemsetAsync(d_nl, 0, sizeof(int), ctx->stream));
         if (lk->nnz) {
@@ -1575,19 +1951,48 @@ extern "C" int hh_links_linked_index(hh_links* lk, const uint8_t* keep, int32_t*
             int grid = (int)(blocks < (int64_t)hh_grid(ctx, 8) ? blocks : (int64_t)hh_grid(ctx, 8));
             HH_LAUNCH(ctx, hh_k_touch, grid, 256, 0, lk->d_compact, lk->nnz, lk->d_keep, d_touch);
         }
-        HH_LAUNCH(ctx, hh_k_rank_touch, (lk->n_ctg + 255) / 256, 256, 0, d_touch, lk->n_ctg, lk->d_index, d_nl);
+        HH_LAUNCH(ctx, hh_k_rank_init, nb, HH_RADIX_TILE, 0, d_touch, n, d_key[0], d_val[0], d_nl);
+        for (int pass = 0; pass < HH_RADIX_PASSES; ++pass) {
+            const int src = pass & 1;
+            HH_LAUNCH(ctx, hh_k_radix_hist, nb, HH_RADIX_TILE, 0, d_key[src], n, 8 * pass, d_cnt);
+            HH_CHECK(hh_exclusive_scan_i32(ctx, d_cnt, d_off, nb * 256));
+            HH_LAUNCH(ctx, hh_k_radix_scatter, nb, HH_RADIX_TILE, 0, d_key[src], d_val[src], n, 8 * pass, d_off, d_key[src ^ 1],
+                      d_val[src ^ 1]);
+        }
+        HH_LAUNCH(ctx, hh_k_rank_index, (n + 255) / 256, 256, 0, d_val[HH_RADIX_PASSES & 1], n, d_nl, lk->d_index);
         HH_CUDA(cudaMemcpyAsync(ctx->h_scratch + 8, d_nl, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
         if (index)
-            HH_CUDA(cudaMemcpyAsync(index, lk->d_index, (size_t)lk->n_ctg * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+            HH_CUDA(cudaMemcpyAsync(index, lk->d_index, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
         HH_CUDA(cudaStreamSynchronize(ctx->stream));
         lk->n_linked = *reinterpret_cast<int*>(ctx->h_scratch + 8);
         return HH_OK;
     }();
     hh_dfree(d_touch);
+    for (int b = 0; b < 2; ++b) {
+        hh_dfree(d_key[b]);
+        hh_dfree(d_val[b]);
+    }
+    hh_dfree(d_cnt);
+    hh_dfree(d_off);
     HH_CHECK(rc);
+    lk->index_keep->assign(keep, keep + n);
+    lk->index_valid = true;
     if (n_linked) *n_linked = lk->n_linked;
     return HH_OK;
 }
+
+// the first-seen index for `keep` on the device (d_index, d_keep): the one hh_links_linked_index left there when it was
+// computed for the same mask and entry list, else computed now
+int hh_links_index_for(hh_links* lk, const uint8_t* keep, int32_t* n_linked) {
+    if (lk->index_valid && memcmp(lk->index_keep->data(), keep, (size_t)lk->n_ctg) == 0) {
+        *n_linked = lk->n_linked;
+        return HH_OK;
+    }
+    return hh_links_linked_index(lk, keep, nullptr, n_linked);
+}
+
+// d_index was changed in place (the matrix build appends the tail fragments to it)
+void hh_links_index_invalidate(hh_links* lk) { lk->index_valid = false; }
 
 extern "C" int hh_links_destroy(hh_links* lk) {
     if (!lk) return HH_OK;
@@ -1617,6 +2022,7 @@ extern "C" int hh_links_destroy(hh_links* lk) {
     hh_dfree(lk->d_keep);
     links_free_partsets(lk);
     delete lk->psets;
+    delete lk->index_keep;
     delete lk;
     return HH_OK;
 }

@@ -105,9 +105,9 @@ extern "C" int hh_matrix_from_links(hh_links* lk, const uint8_t* keep, const int
     hh_ctx* ctx = hh_links_ctx(lk);
     HH_CUDA(cudaSetDevice(ctx->device));
     const int n_ctg = hh_links_n_ctg(lk);
-    // (re)compute the first-seen indices for this keep mask
+    // the first-seen indices for this keep mask (reused when hh_links_linked_index has just computed them)
     int32_t n_linked = 0;
-    HH_CHECK(hh_links_linked_index(lk, keep, nullptr, &n_linked));
+    HH_CHECK(hh_links_index_for(lk, keep, &n_linked));
     int32_t* d_index = hh_links_index_dev(lk, &n_linked);
     const uint8_t* d_keep = hh_links_keep_dev(lk);
     const int n = n_linked + n_tail;
@@ -122,6 +122,7 @@ extern "C" int hh_matrix_from_links(hh_links* lk, const uint8_t* keep, const int
         if (n_tail) {
             HH_CHECK(hh_dmalloc(&d_tail, (size_t)n_tail));
             HH_CUDA(cudaMemcpyAsync(d_tail, tail, (size_t)n_tail * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+            hh_links_index_invalidate(lk);
             HH_LAUNCH(ctx, hh_k_set_tail, (n_tail + 255) / 256, 256, 0, d_tail, n_tail, n_linked, d_keep, d_index, n_ctg, d_err);
         }
         HH_LAUNCH(ctx, hh_k_check_index, (n_ctg + 255) / 256, 256, 0, d_index, d_keep, n_ctg, n, d_err);

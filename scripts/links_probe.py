@@ -1,5 +1,6 @@
 """Link-counting probe at C3 (50k contigs / 200M pairs): wall / device time of add and finish for the direct and the
-partitioned engines.  Run under `ncu --metrics gpu__time_duration.sum` for the per-kernel launch list."""
+partitioned engines.  PROFILE=1 adds one partitioned pass (count + index + matrix) under torch.profiler and prints its
+per-kernel device times."""
 import os
 import sys
 import time
@@ -38,3 +39,18 @@ for mode in os.environ.get("MODES", "0,1").split(","):
               round(1e3 * (t3 - t2), 2), "nnz", info.nnz_full, "slots", info.table_slots, flush=True)
         mat.close()
         tab.close()
+
+if os.environ.get("PROFILE"):
+    from torch.profiler import ProfilerActivity, profile
+    os.environ["HH_LINKS_PARTITION"] = "1"
+    keep = np.ones(asm.n, np.uint8)
+    with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
+        tab = LinkTable(ctx, asm.lengths, rank, in_nx, 500000, capacity_hint=int(0.45 * pairs))
+        tab.add(rec, asynchronous=True)
+        tab.finish()
+        index, _ = tab.linked_index(keep)
+        mat = tab.to_matrix(keep, np.nonzero(index < 0)[0].astype(np.int32))
+        ctx.sync()
+    print(prof.key_averages().table(sort_by="cuda_time_total", row_limit=30, max_name_column_width=60), flush=True)
+    mat.close()
+    tab.close()
