@@ -10,7 +10,7 @@
 //
 // Precision.  The reference multiplies fp32 by fp32.  Tensor cores take bf16, so each operand is split into bf16
 // "planes" whose sum is the fp32 value EXACTLY:
-//   A = C      link counts are integers: <= 256 -> one plane, < 65536 -> two, anything else (weights) three;
+//   A = C      integer link counts: min(count, clip) in one plane, the excess as a sparse correction; anything else three;
 //   B = M0     three planes (8 + 8 + 8 significant bits).
 // A bf16 x bf16 product is exact in fp32, so the passes (plane_a, plane_b) below reproduce the fp32 product up to
 // dropped terms of relative size 2^-24.  The accumulation inside the tensor core is not IEEE round-to-nearest, so a
@@ -191,11 +191,10 @@ struct hh_gemm_args {
     const float* inv_s;    // 1 / column sum
     float out_scale;       // applied instead when inv_s == NULL
     int accumulate;        // 1: the epilogue adds to what the output holds (K range processed in several launches)
-    int split_lo;          // 1: passes with a low-order plane accumulate in their own TMEM buffer over the whole tile (see kernel)
     uint32_t idesc_fmt;    // operand format bits of the instruction descriptor (bit 7: A is bf16, bit 10: B is bf16)
 };
 
-template <int CG, bool SPLIT>
+template <int CG>
 __global__ void __launch_bounds__(HG_THREADS, 1)
 hh_k_syrk(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const hh_gemm_args a) {
     constexpr int BN = 128 * CG;              // tile columns (= TMEM columns per accumulator buffer)
@@ -273,37 +272,29 @@ hh_k_syrk(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
         if (rank == 0 && lane == 0) {
             int s = 0;
             uint32_t ph = 0;
-            uint32_t g = 0;     // running chunk counter: TMEM buffer g & 1, phase (g >> 1) & 1  (split_lo: buffer 0, phase g & 1)
-            constexpr bool split = SPLIT;       // compiled out of the default kernel
+            uint32_t g = 0;     // running chunk counter: TMEM buffer g & 1, phase (g >> 1) & 1
             for (int it = pair; it < a.n_items; it += npairs) {
                 const hh_gemm_item w = a.items[it];
                 int in_chunk = 0;
                 const int total = (w.kb_hi[0] - w.kb_lo[0]) + (w.kb_hi[1] - w.kb_lo[1]);
                 for (int t = 0; t < total; ++t) {
-                    const uint32_t buf = split ? 0u : (g & 1u);
+                    const uint32_t buf = g & 1u;
                     if (in_chunk == 0) {
-                        hg_mbar_wait(hg_smem_u32(&s_tempty[buf]), (split ? (g & 1u) : ((g >> 1) & 1u)) ^ 1u);
+                        hg_mbar_wait(hg_smem_u32(&s_tempty[buf]), ((g >> 1) & 1u) ^ 1u);
                         hg_tc_fence_after();
                     }
                     hg_mbar_wait(hg_smem_u32(&s_full[s]), ph);
                     hg_tc_fence_after();
                     const uint32_t st = smem_base + (uint32_t)s * stage_bytes;
-                    const uint32_t d_hi = tmem_base + buf * (uint32_t)BN;
-                    const uint32_t d_lo = tmem_base + (uint32_t)BN;
-                    uint32_t hi_acc = in_chunk ? 1u : 0u, lo_acc = t ? 1u : 0u;      // 0: the MMA overwrites the accumulator
+                    const uint32_t d = tmem_base + buf * (uint32_t)BN;
+                    uint32_t acc = in_chunk ? 1u : 0u;      // 0: the MMA overwrites the accumulator
                     for (int p = 0; p < a.npass; ++p) {
                         const uint64_t ad = hg_make_desc(st + (uint32_t)a.pa[p] * HG_PLANE_BYTES);
                         const uint64_t bd = hg_make_desc(st + (uint32_t)(a.na + a.pb[p]) * HG_PLANE_BYTES);
-                        const bool lo = split && (a.pa[p] | a.pb[p]) != 0;
 #pragma unroll
                         for (int k = 0; k < 4; ++k) {
-                            if (lo) {
-                                hg_umma<CG>(d_lo, ad + (uint64_t)(2 * k), bd + (uint64_t)(2 * k), IDESC, lo_acc);
-                                lo_acc = 1u;
-                            } else {
-                                hg_umma<CG>(d_hi, ad + (uint64_t)(2 * k), bd + (uint64_t)(2 * k), IDESC, hi_acc);
-                                hi_acc = 1u;
-                            }
+                            hg_umma<CG>(d, ad + (uint64_t)(2 * k), bd + (uint64_t)(2 * k), IDESC, acc);
+                            acc = 1u;
                         }
                     }
                     hg_umma_commit<CG>(hg_smem_u32(&s_empty[s]));      // the stage is free once these MMAs have read it
@@ -328,7 +319,6 @@ hh_k_syrk(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
         const uint32_t lane_addr = ((uint32_t)(quarter * 32) << 16) + (uint32_t)(half * CW);
         const uint32_t tempty0 = (CG == 2) ? hg_mapa(hg_smem_u32(&s_tempty[0]), 0) : hg_smem_u32(&s_tempty[0]);
         uint32_t g = 0;
-        constexpr bool split = SPLIT;
         float acc[CW];
         for (int it = pair; it < a.n_items; it += npairs) {
             const hh_gemm_item w = a.items[it];
@@ -337,21 +327,17 @@ hh_k_syrk(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
 #pragma unroll
             for (int j = 0; j < CW; ++j) acc[j] = 0.f;
             for (int ch = 0; ch < nchunks; ++ch, ++g) {
-                const uint32_t buf = split ? 0u : (g & 1u);
-                hg_mbar_wait(hg_smem_u32(&s_tfull[buf]), split ? (g & 1u) : ((g >> 1) & 1u));
+                const uint32_t buf = g & 1u;
+                hg_mbar_wait(hg_smem_u32(&s_tfull[buf]), (g >> 1) & 1u);
                 hg_tc_fence_after();
-                // split_lo: after the last chunk of the tile the low-order accumulator (second buffer) is added as well
-                const int nsrc = (split && ch + 1 == nchunks) ? 2 : 1;
-                for (int src = 0; src < nsrc; ++src) {
-                    const uint32_t tb = tmem_base + (src ? (uint32_t)BN : buf * (uint32_t)BN) + lane_addr;
+                const uint32_t tb = tmem_base + buf * (uint32_t)BN + lane_addr;
 #pragma unroll
-                    for (int q = 0; q < CW / 32; ++q) {
-                        uint32_t v[32];
-                        hg_tmem_ld32(tb + (uint32_t)(q * 32), v);
-                        hg_tmem_ld_wait();
+                for (int q = 0; q < CW / 32; ++q) {
+                    uint32_t v[32];
+                    hg_tmem_ld32(tb + (uint32_t)(q * 32), v);
+                    hg_tmem_ld_wait();
 #pragma unroll
-                        for (int j = 0; j < 32; ++j) acc[q * 32 + j] = __fadd_rn(acc[q * 32 + j], __uint_as_float(v[j]));
-                    }
+                    for (int j = 0; j < 32; ++j) acc[q * 32 + j] = __fadd_rn(acc[q * 32 + j], __uint_as_float(v[j]));
                 }
                 hg_tc_fence_before();
                 __syncwarp();
@@ -548,9 +534,9 @@ static int hg_env_int(const char* name, int dflt) {
     return (v && *v) ? atoi(v) : dflt;
 }
 
-template <int CG, bool SPLIT>
+template <int CG>
 static int hg_launch(hh_ctx* ctx, const CUtensorMap& tmA, const CUtensorMap& tmB, const hh_gemm_args& a, size_t smem) {
-    auto kern = hh_k_syrk<CG, SPLIT>;
+    auto kern = hh_k_syrk<CG>;
     HH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
@@ -577,7 +563,7 @@ int hh_gemm_cta_group() { return hg_env_int("HH_GEMM_CG", 2) == 1 ? 1 : 2; }
 
 int hh_gemm_run(hh_ctx* ctx, const hh_gemm_operand& A, const hh_gemm_operand& B, const hh_gemm_item* d_items, int n_items, int npass,
                 const int* pa, const int* pb, int chunk_kb, float* out, long long ld, int col_lo, int col_hi, const float* scale,
-                int* stages_out, float out_scale, int split_lo, int accumulate) {
+                int* stages_out, float out_scale, int accumulate) {
     HH_REQUIRE(n_items >= 1 && npass >= 1 && npass <= 8, HH_ERR_ARG, "hh_gemm_run: bad work list");
     CUtensorMap tmA, tmB;
     HH_CHECK(hg_encode(&tmA, (void*)A.base, A.rows, A.kdim, A.ldk, A.plane, A.planes, A.fmt));
@@ -606,22 +592,20 @@ int hh_gemm_run(hh_ctx* ctx, const hh_gemm_operand& A, const hh_gemm_operand& B,
     a.col_hi = col_hi;
     a.inv_s = scale;
     a.out_scale = out_scale;
-    a.split_lo = split_lo;
     a.accumulate = accumulate;
     a.idesc_fmt = (A.fmt == HH_GEMM_BF16 ? (1u << 7) : 0u) | (B.fmt == HH_GEMM_BF16 ? (1u << 10) : 0u);
     const size_t smem = (size_t)stages * stage_bytes + 1024;
-    if (hh_gemm_cta_group() == 2) return split_lo ? hg_launch<2, true>(ctx, tmA, tmB, a, smem) : hg_launch<2, false>(ctx, tmA, tmB, a, smem);
-    return split_lo ? hg_launch<1, true>(ctx, tmA, tmB, a, smem) : hg_launch<1, false>(ctx, tmA, tmB, a, smem);
+    if (hh_gemm_cta_group() == 2) return hg_launch<2>(ctx, tmA, tmB, a, smem);
+    return hg_launch<1>(ctx, tmA, tmB, a, smem);
 }
 
 static const int HG_P1[3][2] = {{0, 0}, {0, 1}, {0, 2}};
-static const int HG_P2[5][2] = {{0, 0}, {0, 1}, {1, 0}, {0, 2}, {1, 1}};
 static const int HG_P3[6][2] = {{0, 0}, {0, 1}, {1, 0}, {0, 2}, {1, 1}, {2, 0}};
 
-// pass list for `na` planes of A against three planes of B: every product of relative size >= 2^-16 (na = 1: exact)
+// pass list for `na` (1 or 3) planes of A against three planes of B: every product of relative size >= 2^-16 (na = 1: exact)
 int hh_gemm_passes(int na, int* pa, int* pb) {
-    const int(*pl)[2] = na == 1 ? HG_P1 : (na == 2 ? HG_P2 : HG_P3);
-    const int np = na == 1 ? 3 : (na == 2 ? 5 : 6);
+    const int(*pl)[2] = na == 1 ? HG_P1 : HG_P3;
+    const int np = na == 1 ? 3 : 6;
     for (int p = 0; p < np; ++p) {
         pa[p] = pl[p][0];
         pb[p] = pl[p][1];
@@ -663,13 +647,9 @@ int hh_gemm_preexpand(hh_ctx* ctx, const hh_matrix* m, int col_lo, int col_hi, f
         int enc = 2;                                             // 0 = exact bf16, 2 = scaled f16
         if (fmt_env && !strcmp(fmt_env, "bf16")) enc = 0;
         if (flags & (1 | 4)) enc = 0;
-        int na = (flags & 1) ? 3 : 1;
+        const int na = (flags & 1) ? 3 : 1;
         const int nb = enc ? 2 : 3;
-        float clip = (flags & 1) ? 3.0e38f : (enc == 2 ? 2048.f : 256.f);
-        if (hg_env_int("HH_GEMM_NA", 0) == 2 && !(flags & 1) && enc == 0) {      // experiment: two planes instead of clipping
-            na = 2;
-            clip = 3.0e38f;
-        }
+        const float clip = (flags & 1) ? 3.0e38f : (enc == 2 ? 2048.f : 256.f);
         const int fmt_a = enc == 2 ? HH_GEMM_F16 : HH_GEMM_BF16, fmt_b = enc ? HH_GEMM_F16 : HH_GEMM_BF16;
         // The K range is cut into equal chunks when the operand planes of the whole range would exceed ~36 GB (150k contigs:
         // 135 GB): planes of one chunk at a time, the epilogue of every chunk after the first adds to M1.  The cut depends on
@@ -694,8 +674,6 @@ int hh_gemm_preexpand(hh_ctx* ctx, const hh_matrix* m, int col_lo, int col_hi, f
             pb[0] = 0;
             pb[1] = 1;
         }
-        const int np_env = hg_env_int("HH_GEMM_NPASS", 0);      // experiments only: fewer passes = lower precision
-        if (np_env >= 1 && np_env < npass) npass = np_env;
         // k-blocks accumulated in TMEM between two drains: the tensor core's accumulate truncates, so the bias grows with the
         // number of accumulations (4 MMAs per k-block and pass).
         // Measured at 50k contigs (one B200; GEMM time / max and mean relative error against the exact product), two f16 passes:
@@ -703,11 +681,10 @@ int hh_gemm_preexpand(hh_ctx* ctx, const hh_matrix* m, int col_lo, int col_hi, f
         // every drain costs 0.5-2k clocks of tensor-pipe time, so longer chunks are faster -- but on dense inputs (every product
         // of similar size) the bias of 64 truncating accumulations reaches 2.5e-6.  Three k-blocks = 24 accumulations, the
         // same as three bf16 passes drained every second k-block, keeps every test input below 2e-6.
-        // HH_GEMM_SPLIT=1 (experiment): the low-order pass (2^-11 of the result) gets the second TMEM buffer for the whole
-        // tile and only the high-order pass is chunked -- bias-free (mean -1.4e-10) but single-buffered: 244 ms against 211 ms
-        // at chunk 8 on the same device.
-        const int split = (enc && hg_env_int("HH_GEMM_SPLIT", 0)) ? 1 : 0;
-        const int chunk = hg_env_int("HH_GEMM_CHUNK", npass > 3 ? 1 : (npass == 3 ? 2 : (split ? 8 : 3)));
+        // Giving the low-order pass (2^-11 of the result) the second TMEM buffer for the whole tile and chunking only the
+        // high-order pass was measured bias-free (mean -1.4e-10) but, single-buffered, slower: 244 ms against 211 ms at
+        // chunk 8 on the same device.
+        const int chunk = hg_env_int("HH_GEMM_CHUNK", npass > 3 ? 1 : (npass == 3 ? 2 : 3));
         int stages = 0;
         float densify_ms = 0.f, gemm_ms = 0.f;
         const float stats_ms = 0.f;                              // column sums + value statistics: a fraction of a millisecond
@@ -732,8 +709,7 @@ int hh_gemm_preexpand(hh_ctx* ctx, const hh_matrix* m, int col_lo, int col_hi, f
             hh_gemm_operand A = {d_A, na, n, (int)(k1 - k0), kw, plane_c, fmt_a};
             hh_gemm_operand B = {d_B, nb, n, (int)(k1 - k0), kw, plane_c, fmt_b};
             HH_CUDA(cudaEventRecord(ev[1], ctx->stream));
-            HH_CHECK(hh_gemm_run(ctx, A, B, d_items, n_items, npass, pa, pb, chunk, d_m1, ld, col_lo, col_hi, d_inv, &stages, 1.0f, split,
-                                 kc > 0 ? 1 : 0));
+            HH_CHECK(hh_gemm_run(ctx, A, B, d_items, n_items, npass, pa, pb, chunk, d_m1, ld, col_lo, col_hi, d_inv, &stages, 1.0f, kc > 0 ? 1 : 0));
             HH_CUDA(cudaEventRecord(ev[2], ctx->stream));
             HH_CUDA(cudaStreamSynchronize(ctx->stream));         // items_c is rewritten for the next chunk
             float t0 = 0.f, t1 = 0.f;

@@ -46,13 +46,11 @@ int hh_gemm_preexpand(hh_ctx* ctx, const hh_matrix* m, int col_lo, int col_hi, f
                       int n_items, hh_gemm_stats* st);
 // the GEMM itself on prepared operands: D tiles listed in d_items (device), written to out (column-major, leading dimension
 // ld, columns [col_lo, col_hi)), each element multiplied by scale[c] when scale != NULL.  The pass list multiplies plane
-// pa[p] of A with plane pb[p] of B.  split_lo = 1: passes that involve a plane > 0 accumulate in a second TMEM buffer over
-// the whole tile instead of sharing the chunked accumulator (only sound when those planes are <= 2^-11 of the value).
-// accumulate = 1: the epilogue adds to the values `out` holds (the K range of a product processed in several launches).
+// pa[p] of A with plane pb[p] of B.  accumulate = 1: the epilogue adds to the values `out` holds (the K range of a product processed in several launches).
 // Asynchronous on the context's stream.
 int hh_gemm_run(hh_ctx* ctx, const hh_gemm_operand& A, const hh_gemm_operand& B, const hh_gemm_item* d_items, int n_items, int npass,
                 const int* pa, const int* pb, int chunk_kb, float* out, long long ld, int col_lo, int col_hi, const float* scale,
-                int* stages_out, float out_scale, int split_lo, int accumulate);
+                int* stages_out, float out_scale, int accumulate);
 int hh_gemm_cta_group();
 int hh_gemm_passes(int na, int* pa, int* pb);
 

@@ -17,7 +17,6 @@
 //
 //   SRC_CSC     scatter an unsorted CSC column            (dict_to_matrix output, 366-368)
 //   SRC_PRODUCT expansion, A.B column product             (mkl_matrix_power, 2017-2023)
-//   SRC_DENSE   stream a column of the dense pre-expanded M1 (iteration 0 skips expansion, 2030)
 //   EPI_NORM    column L1 normalise (sklearn normalize, 2144) or raw copy (canonical CSC)
 //   EPI_DUMP    write the accumulator as a dense column    (pre-expansion result, 2146-2149)
 //   EPI_PRUNE   inflate + normalise (2038), prune + keep first max + normalise (1987-2014),
@@ -54,7 +53,7 @@ __device__ __forceinline__ float hh_inflate(float x, float rf, int mode) {
     }
 }
 
-enum { SRC_CSC = 0, SRC_PRODUCT = 1, SRC_DENSE = 2 };
+enum { SRC_CSC = 0, SRC_PRODUCT = 1 };
 enum { EPI_NORM = 0, EPI_DUMP = 1, EPI_PRUNE = 2 };
 // Link counts above the clip threshold of the tensor-core encoding (hh_gemm_stats.clip: 2048 for an f16 plane, 256 for a bf16
 // plane) are split: min(x, clip) goes through the GEMM as ONE exact plane, the rest through two small Gustavson corrections
@@ -77,7 +76,7 @@ struct hh_colargs {
     int do_conv;
     int track;                   // product + prune only: keep the dirty-chunk bitmap (sparse columns)
     // cluster-contiguous relabelling ("perm space"): new index = perm[original index], orig = inverse
-    const int* perm;             // SRC_DENSE / SRC_CSC(slot source): scatter rows through perm
+    const int* perm;             // SRC_CSC(slot source): scatter rows through perm
     const int* orig;             // original index of every (new) row: tie-break of the first maximum; source column lookup
     int slot_src;                // SRC_CSC: read the column from slotted matrix B (column orig[j] when orig != NULL) instead of a CSC
     const int* ncols_ptr;        // optional: number of columns to process is read from device memory (overflow list)
@@ -132,7 +131,7 @@ __global__ void __launch_bounds__(W * 32) hh_k_col(const hh_colargs a) {
         const int jj = s_col;
         if (jj >= ncols_run) break;
         const int j = a.order ? a.order[jj] : (a.col_lo + jj);
-        const int jsrc = (a.orig && (SRC == SRC_DENSE || (SRC == SRC_CSC && a.slot_src))) ? a.orig[j] : j;   // source column
+        const int jsrc = (a.orig && SRC == SRC_CSC && a.slot_src) ? a.orig[j] : j;   // source column
         const int jloc = jsrc - a.col_lo;       // position inside the owned (dense) column block
         uint64_t dirty = 0ull;
 
@@ -151,41 +150,6 @@ __global__ void __launch_bounds__(W * 32) hh_k_col(const hh_colargs a) {
                 for (int64_t p = p0 + threadIdx.x; p < p1; p += W * 32) atomicAdd(&acc[a.csc_row[p]], a.csc_val[p]);
             }
             __syncthreads();
-            dirty = ALL;
-        } else if (SRC == SRC_DENSE) {
-            // stream the dense column: 128-bit loads, all issued before the first store (rows >= n of
-            // the padded column are zeros written by the pre-expansion)
-            const float4* __restrict__ col4 = reinterpret_cast<const float4*>(a.dense_in + (size_t)jloc * (size_t)a.ld);
-            const int ld4 = (int)(a.ld >> 2);
-            if (a.perm) {
-                // perm space: source row r lands in accumulator row perm[r] (any warp's tile) -> block-wide load
-                const int n4 = (a.n + 3) >> 2;
-                for (int r4 = threadIdx.x; r4 < n4; r4 += W * 32) {
-                    const float4 x = hh_ld_stream_f4(col4 + r4);
-                    const int r = r4 << 2;
-                    if (r < a.n) acc[a.perm[r]] = x.x;
-                    if (r + 1 < a.n) acc[a.perm[r + 1]] = x.y;
-                    if (r + 2 < a.n) acc[a.perm[r + 2]] = x.z;
-                    if (r + 3 < a.n) acc[a.perm[r + 3]] = x.w;
-                }
-                __syncthreads();
-            } else {
-            const int r4_0 = (tile0 >> 2) + lane, r4_end = (tile0 + T) >> 2;
-            for (int r4 = r4_0; r4 < r4_end; r4 += 128) {
-                float4 x[4];
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const int rr = r4 + q * 32;
-                    x[q] = (rr < r4_end && rr < ld4) ? hh_ld_stream_f4(col4 + rr) : make_float4(0.f, 0.f, 0.f, 0.f);
-                }
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const int rr = r4 + q * 32;
-                    if (rr < r4_end) reinterpret_cast<float4*>(acc)[rr] = x[q];
-                }
-            }
-            }
-            __syncwarp();
             dirty = ALL;
         } else {
             // Gustavson expansion restricted to this warp's row block.  The B entries of column j are
@@ -473,43 +437,6 @@ __global__ void __launch_bounds__(W * 32) hh_k_col(const hh_colargs a) {
             int cnt = 0;
             float vbest = 0.f;
             int kbest = 0x7fffffff, obest = 0x7fffffff;     // obest: ORIGINAL row index of kbest (first maximum = lowest original row)
-            if (SRC == SRC_DENSE && !a.do_conv && S1 != 0.0) {
-                // Dense iteration 0: every one of the n rows is stored, but only entries with x1 = fp32(fp64(y) / S1) >= pruning
-                // can survive (at most 1/pruning of them).  The exact fp64 quotient is taken for the candidates
-                // y >= 0.999 * pruning * S1 only; the others are provably below the threshold, keep the fp32 product
-                // y * (1 / S1) (never stored) and take part in the maximum through their exact ordering by y.
-                const float thr = (float)(0.999 * (double)p32 * S1);
-                const float inv1 = (float)(1.0 / S1);
-                float ybest = 0.f;
-                HH_FOR_DIRTY_ROWS({
-                    const float y = acc[k];
-                    if (y != 0.f) {
-                        float x1;
-                        if (y >= thr) {
-                            x1 = (float)((double)y / S1);
-                            if (x1 >= p32 && x1 > 0.f) {
-                                cnt++;
-                                s2 += (double)x1;
-                            }
-                        } else {
-                            x1 = fminf(y * inv1, 0.9995f * p32);     // strictly below the threshold whatever the rounding
-                        }
-                        acc[k] = x1;
-                        if (y > ybest) {                // rows ascend inside a lane: the first maximum wins
-                            // two different y may round to the same x1: then the earlier row stays (first maximum of x1)
-                            bool take = true;
-                            if (y <= ybest * 1.0000005f) take = (float)((double)y / S1) > (float)((double)ybest / S1);
-                            if (take) {
-                                ybest = y;
-                                kbest = k;
-                            }
-                        }
-                    }
-                })
-                // exact quotient of the lane's maximum (x1 is monotone in y)
-                vbest = (ybest > 0.f) ? (float)((double)ybest / S1) : 0.f;
-                obest = (a.orig && kbest != 0x7fffffff) ? a.orig[kbest] : kbest;
-            } else {
             HH_FOR_DIRTY_ROWS({
                 const float y = acc[k];
                 if (y != 0.f) {
@@ -532,7 +459,6 @@ __global__ void __launch_bounds__(W * 32) hh_k_col(const hh_colargs a) {
                     }
                 }
             })
-            }
             s2 = hh_warp_sum(s2);
             cnt = hh_warp_sum(cnt);
 #pragma unroll
@@ -1556,14 +1482,12 @@ struct hh_mcl {
     int* d_counter;
     unsigned long long* d_stats;   // [0] nnz [1] products [2] delta bits [3] err
     int64_t nnz_m0, preexp_products;
-    int flat, l2pf;                // expansion inner-loop variant / L2 prefetch (HH_MCL_FLAT, HH_MCL_L2PF)
     int32_t own_lo, own_hi;        // the column block given to hh_mcl_create (dense M1 block); col_lo/col_hi = active block
     int* d_order;                  // [ncols] processing order for the next expansion
     int* d_cnt;                    // [2n] histogram + cursors
-    int use_small;                 // warp-per-column kernel for nearly converged iterates (HH_MCL_SMALL)
+    int use_small;                 // warp-per-column kernel for nearly converged iterates
     int* d_bigcount;
-    // cluster-contiguous relabelling + windowed expansion (HH_MCL_WINDOW)
-    int use_window;
+    int use_window;                // cluster-contiguous relabelling + windowed expansion
     bool perm_valid;               // perm / lists below are built (once per hh_mcl, from the first pruned iterate)
     bool perm_space;               // the iterates it[] are stored in new (perm) indices
     int last_step_it;              // iteration number of the pending / last committed step
@@ -1625,11 +1549,16 @@ static int env_int(const char* name, int dflt) {
     return (v && *v) ? atoi(v) : dflt;
 }
 
+// link count from which an edge of the input matrix is "strong": the components of the strong-link graph order the columns
+// of the pre-expansion (hh_k_cc_hook_csc)
+static constexpr float HH_PREORDER_STRONG = 10.f;
+// largest component (rows) that gets a window: the relabelling and expansion window kernels and the block-diagonal GEMM
+// take these; larger components stay on the n-row column kernel
+static constexpr int HH_WINDOW_MAX = 8192;
+
 static hh_geom geom_for(hh_ctx* ctx, int n) {
     hh_geom g;
     g.W = (n <= 12288) ? 8 : (n <= 28672 ? 16 : 32);
-    const int wo = env_int("HH_MCL_W", 0);       // tuning override: row blocks per column = warps per CTA
-    if (wo == 8 || wo == 16 || wo == 32) g.W = wo;
     int T = (n + g.W - 1) / g.W;
     T = (T + 31) & ~31;
     g.T = T;
@@ -1716,20 +1645,20 @@ __device__ __noinline__ float hh_it0_x1(float x, double S1, float rf, int sq) {
     return (float)((double)y / S1);
 }
 
-// NW warps per CTA and 32 / NW CTAs per SM.  With 8-warp CTAs 592 columns (118 MB, the whole L2) are in flight and ncu shows
+// 8 warps per CTA and 4 CTAs per SM: 592 columns (118 MB, the whole L2) are in flight and ncu shows
 // all three passes in DRAM (29.6 GB read, L2 hit 4 %) -- but fewer, larger CTAs (59 / 30 MB in flight) are not faster:
-// 10.1 / 10.5 / 11.6 ms for NW = 8 / 16 / 32 at r = 2.0 on the same device.  The kernel is bound by instruction issue
-// (1.0e10 warp instructions, issue slots 61 % busy), not by where the re-reads come from.  HH_MCL_IT0_WARPS selects the shape.
-// QUEUE: the candidates of passes 2 and 3 (a few percent of the elements) are first collected in a per-warp shared-memory
+// 10.1 / 10.5 / 11.6 ms for 8 / 16 / 32 warps at r = 2.0 on the same device.  The kernel is bound by instruction issue
+// (1.0e10 warp instructions, issue slots 61 % busy), not by where the re-reads come from.
+// The candidates of passes 2 and 3 (a few percent of the elements) are first collected in a per-warp shared-memory
 // queue and then evaluated 32 at a time.  Evaluating them where they are found costs one call of hh_it0_x1 (pow + fp64
 // division, ~100 instructions) per warp and element slot that holds at least one candidate -- with 1-2 % candidates that
 // is every second slot, executed with one or two active lanes: 7.5e9 of the kernel's 1.0e10 warp instructions (ncu).
-template <int W, bool SQ, int NW, bool QUEUE>      // SQ: any of the multiplicative modes (no powf in the streaming loop)
-__global__ void __launch_bounds__(NW * 32, 32 / NW) hh_k_iter0(const hh_colargs a) {
-    constexpr int HH_IT0_WARPS = NW;
+constexpr int HH_IT0_WARPS = 8;
+template <int W, bool SQ>      // SQ: any of the multiplicative modes (no powf in the streaming loop)
+__global__ void __launch_bounds__(HH_IT0_WARPS * 32, 32 / HH_IT0_WARPS) hh_k_iter0(const hh_colargs a) {
     constexpr int QCAP = 256;                       // queue entries per warp (a trip adds at most 128)
-    __shared__ float s_qx[QUEUE ? NW : 1][QUEUE ? QCAP : 1];
-    __shared__ unsigned s_qr[QUEUE ? NW : 1][QUEUE ? QCAP : 1];
+    __shared__ float s_qx[HH_IT0_WARPS][QCAP];
+    __shared__ unsigned s_qr[HH_IT0_WARPS][QCAP];
     const unsigned lt_mask = (1u << (threadIdx.x & 31)) - 1u;
     // HH_IT0_WARPS warps per CTA (several CTAs per SM keep loads of other columns in flight across the reductions); warp v
     // handles the row blocks v, v + HH_IT0_WARPS, ... of the slotted format (W blocks of T rows)
@@ -1812,7 +1741,7 @@ __global__ void __launch_bounds__(NW * 32, 32 / NW) hh_k_iter0(const hh_colargs 
                 for (int i0 = 0; i0 < qn; i0 += 32) {
                     const int i = i0 + lane;
                     if (i < qn) {
-                        const float x1 = hh_it0_x1(s_qx[QUEUE ? wv : 0][QUEUE ? i : 0], S1, rf, sq);
+                        const float x1 = hh_it0_x1(s_qx[wv][i], S1, rf, sq);
                         if (x1 >= p32 && x1 > 0.f) {
                             cnt++;
                             s2 += (double)x1;
@@ -1822,8 +1751,8 @@ __global__ void __launch_bounds__(NW * 32, 32 / NW) hh_k_iter0(const hh_colargs 
                 __syncwarp();
                 qn = 0;
             };
-            for (int r4 = r4_lo + lane - (QUEUE ? lane : 0); r4 < r4_hi; r4 += 128) {
-                const int r4l = QUEUE ? r4 + lane : r4;      // QUEUE: warp-uniform trip count, the lane offset is added here
+            for (int r4 = r4_lo; r4 < r4_hi; r4 += 128) {
+                const int r4l = r4 + lane;      // warp-uniform trip count, the lane offset is added here
                 float4 x[4];
 #pragma unroll
                 for (int q = 0; q < 4; ++q) x[q] = (r4l + 32 * q < r4_hi) ? hh_ld_stream_f4(col4 + r4l + 32 * q) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -1832,25 +1761,17 @@ __global__ void __launch_bounds__(NW * 32, 32 / NW) hh_k_iter0(const hh_colargs 
                     const float xv[4] = {x[q].x, x[q].y, x[q].z, x[q].w};
 #pragma unroll
                     for (int c = 0; c < 4; ++c) {
-                        if (QUEUE) {
-                            const bool cand = xv[c] >= xthr;
-                            const unsigned bal = __ballot_sync(HH_FULL_MASK, cand);
-                            if (bal) {
-                                if (cand) s_qx[QUEUE ? wv : 0][QUEUE ? qn + __popc(bal & lt_mask) : 0] = xv[c];
-                                qn += __popc(bal);
-                            }
-                        } else if (xv[c] >= xthr) {
-                            const float x1 = hh_it0_x1(xv[c], S1, rf, sq);
-                            if (x1 >= p32 && x1 > 0.f) {
-                                cnt++;
-                                s2 += (double)x1;
-                            }
+                        const bool cand = xv[c] >= xthr;
+                        const unsigned bal = __ballot_sync(HH_FULL_MASK, cand);
+                        if (bal) {
+                            if (cand) s_qx[wv][qn + __popc(bal & lt_mask)] = xv[c];
+                            qn += __popc(bal);
                         }
                     }
-                    if (QUEUE && qn > QCAP - 128) drain2();
+                    if (qn > QCAP - 128) drain2();
                 }
             }
-            if (QUEUE && qn > 0) drain2();
+            if (qn > 0) drain2();
             cnt = hh_warp_sum(cnt);
             if (lane == 0) s_c[b] = cnt;
         }
@@ -1894,91 +1815,53 @@ __global__ void __launch_bounds__(NW * 32, 32 / NW) hh_k_iter0(const hh_colargs 
             if (mine == 0) continue;
             const int r4_lo = (b * T) >> 2, r4_hi = min(((b + 1) * T) >> 2, ld4);
             int off = base;
-            if (QUEUE) {
-                // candidates into the queue in row order (lane-major, then the four rows of a lane), survivors out of it in the
-                // same order: position = off + rank among the survivors of the drained batch
-                int qn = 0;
-                auto drain3 = [&]() {
-                    __syncwarp();
-                    for (int i0 = 0; i0 < qn; i0 += 32) {
-                        const int i = i0 + lane;
-                        float x1 = 0.f;
-                        unsigned row = 0u;
-                        if (i < qn) {
-                            x1 = hh_it0_x1(s_qx[QUEUE ? wv : 0][QUEUE ? i : 0], S1, rf, sq);
-                            row = s_qr[QUEUE ? wv : 0][QUEUE ? i : 0];
-                        }
-                        const bool sv = (i < qn) && x1 >= p32 && x1 > 0.f;
-                        const unsigned bal = __ballot_sync(HH_FULL_MASK, sv);
-                        if (sv) {
-                            const int pos = off + __popc(bal & lt_mask);
-                            if (pos < a.out.cap) oent[pos] = make_uint2(row, __float_as_uint((float)((double)x1 / S2)));
-                        }
-                        off += __popc(bal);
+            // candidates into the queue in row order (lane-major, then the four rows of a lane), survivors out of it in the
+            // same order: position = off + rank among the survivors of the drained batch
+            int qn = 0;
+            auto drain3 = [&]() {
+                __syncwarp();
+                for (int i0 = 0; i0 < qn; i0 += 32) {
+                    const int i = i0 + lane;
+                    float x1 = 0.f;
+                    unsigned row = 0u;
+                    if (i < qn) {
+                        x1 = hh_it0_x1(s_qx[wv][i], S1, rf, sq);
+                        row = s_qr[wv][i];
                     }
-                    __syncwarp();
-                    qn = 0;
-                };
-                for (int r4 = r4_lo; r4 < r4_hi; r4 += 32) {
-                    const int rr = r4 + lane;
-                    float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
-                    if (rr < r4_hi) x = hh_ld_stream_f4(col4 + rr);
-                    const float xv[4] = {x.x, x.y, x.z, x.w};
-                    const bool c0 = xv[0] >= xthr, c1 = xv[1] >= xthr, c2 = xv[2] >= xthr, c3 = xv[3] >= xthr;
-                    const unsigned b0 = __ballot_sync(HH_FULL_MASK, c0), b1 = __ballot_sync(HH_FULL_MASK, c1);
-                    const unsigned b2 = __ballot_sync(HH_FULL_MASK, c2), b3 = __ballot_sync(HH_FULL_MASK, c3);
-                    if ((b0 | b1 | b2 | b3) == 0u) continue;
-                    int pos = qn + __popc(b0 & lt_mask) + __popc(b1 & lt_mask) + __popc(b2 & lt_mask) + __popc(b3 & lt_mask);
-                    const bool cc[4] = {c0, c1, c2, c3};
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        if (cc[q]) {
-                            s_qx[QUEUE ? wv : 0][QUEUE ? pos : 0] = xv[q];
-                            s_qr[QUEUE ? wv : 0][QUEUE ? pos : 0] = (unsigned)((rr << 2) + q);
-                            pos++;
-                        }
+                    const bool sv = (i < qn) && x1 >= p32 && x1 > 0.f;
+                    const unsigned bal = __ballot_sync(HH_FULL_MASK, sv);
+                    if (sv) {
+                        const int pos = off + __popc(bal & lt_mask);
+                        if (pos < a.out.cap) oent[pos] = make_uint2(row, __float_as_uint((float)((double)x1 / S2)));
                     }
-                    qn += __popc(b0) + __popc(b1) + __popc(b2) + __popc(b3);
-                    if (qn > QCAP - 128) drain3();
+                    off += __popc(bal);
                 }
-                if (qn > 0) drain3();
-                continue;
-            }
-            for (int r4 = r4_lo; r4 < r4_hi; r4 += 32) {            // one float4 per lane and trip: rows ascend with the lane
+                __syncwarp();
+                qn = 0;
+            };
+            for (int r4 = r4_lo; r4 < r4_hi; r4 += 32) {
                 const int rr = r4 + lane;
                 float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (rr < r4_hi) x = hh_ld_stream_f4(col4 + rr);
                 const float xv[4] = {x.x, x.y, x.z, x.w};
-                float keep[4];
-                int c = 0;
+                const bool c0 = xv[0] >= xthr, c1 = xv[1] >= xthr, c2 = xv[2] >= xthr, c3 = xv[3] >= xthr;
+                const unsigned b0 = __ballot_sync(HH_FULL_MASK, c0), b1 = __ballot_sync(HH_FULL_MASK, c1);
+                const unsigned b2 = __ballot_sync(HH_FULL_MASK, c2), b3 = __ballot_sync(HH_FULL_MASK, c3);
+                if ((b0 | b1 | b2 | b3) == 0u) continue;
+                int pos = qn + __popc(b0 & lt_mask) + __popc(b1 & lt_mask) + __popc(b2 & lt_mask) + __popc(b3 & lt_mask);
+                const bool cc[4] = {c0, c1, c2, c3};
 #pragma unroll
                 for (int q = 0; q < 4; ++q) {
-                    keep[q] = 0.f;
-                    if (xv[q] >= xthr) {
-                        const float x1 = hh_it0_x1(xv[q], S1, rf, sq);
-                        if (x1 >= p32 && x1 > 0.f) {
-                            keep[q] = x1;
-                            c++;
-                        }
-                    }
-                }
-                if (__ballot_sync(HH_FULL_MASK, c > 0) == 0u) continue;
-                int inc = c;
-#pragma unroll
-                for (int o = 1; o < 32; o <<= 1) {
-                    const int tt = __shfl_up_sync(HH_FULL_MASK, inc, o);
-                    if (lane >= o) inc += tt;
-                }
-                int pos = off + inc - c;
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    if (keep[q] > 0.f) {
-                        if (pos < a.out.cap) oent[pos] = make_uint2((unsigned)((rr << 2) + q), __float_as_uint((float)((double)keep[q] / S2)));
+                    if (cc[q]) {
+                        s_qx[wv][pos] = xv[q];
+                        s_qr[wv][pos] = (unsigned)((rr << 2) + q);
                         pos++;
                     }
                 }
-                off += __shfl_sync(HH_FULL_MASK, inc, 31);
+                qn += __popc(b0) + __popc(b1) + __popc(b2) + __popc(b3);
+                if (qn > QCAP - 128) drain3();
             }
+            if (qn > 0) drain3();
         }
         if (threadIdx.x == 0) {
             a.out.blk[(size_t)j * (W + 1) + W] = min(total, a.out.cap);
@@ -1990,10 +1873,9 @@ __global__ void __launch_bounds__(NW * 32, 32 / NW) hh_k_iter0(const hh_colargs 
     if (threadIdx.x == 0 && nnz_acc) atomicAdd(a.stats + 0, nnz_acc);
 }
 
-template <int W, int NW, bool QUEUE>
-static int launch_iter0_wn(hh_ctx* ctx, hh_colargs& a) {
-    constexpr int HH_IT0_WARPS = NW;
-    auto kern = (a.inflate_square != HH_INFL_POW) ? hh_k_iter0<W, true, NW, QUEUE> : hh_k_iter0<W, false, NW, QUEUE>;
+template <int W>
+static int launch_iter0_w(hh_ctx* ctx, hh_colargs& a) {
+    auto kern = (a.inflate_square != HH_INFL_POW) ? hh_k_iter0<W, true> : hh_k_iter0<W, false>;
     int per_sm = 0;
     HH_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, HH_IT0_WARPS * 32, 0));
     if (per_sm < 1) per_sm = 1;
@@ -2003,16 +1885,6 @@ static int launch_iter0_wn(hh_ctx* ctx, hh_colargs& a) {
     HH_CUDA(cudaMemsetAsync(a.counter, 0, sizeof(int), ctx->stream));
     HH_LAUNCH(ctx, kern, grid, HH_IT0_WARPS * 32, 0, a);
     return HH_OK;
-}
-
-template <int W>
-static int launch_iter0_w(hh_ctx* ctx, hh_colargs& a) {
-    if (env_int("HH_MCL_IT0_QUEUE", 1)) return launch_iter0_wn<W, 8, true>(ctx, a);      // candidates evaluated 32 at a time
-    switch (env_int("HH_MCL_IT0_WARPS", 8)) {
-        case 16: return launch_iter0_wn<W, 16, false>(ctx, a);
-        case 32: return launch_iter0_wn<W, 32, false>(ctx, a);
-        default: return launch_iter0_wn<W, 8, false>(ctx, a);
-    }
 }
 
 static int launch_iter0(hh_ctx* ctx, const hh_geom& g, hh_colargs& a) {
@@ -2158,7 +2030,7 @@ static int slot_from_csc_fast(hh_ctx* ctx, const hh_geom& g, int* d_counter, uns
     *done = false;
     const int nw_pad = (((m->n + 31) >> 5) + 255) & ~255;
     const size_t smem = (size_t)nw_pad * 2 * sizeof(uint32_t);
-    if (smem + 1024 > ctx->smem_optin || !env_int("HH_MCL_NORM_FAST", 1)) return HH_OK;
+    if (smem + 1024 > ctx->smem_optin) return HH_OK;
     auto kern = hh_k_slot_from_csc;
     HH_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
@@ -2403,23 +2275,19 @@ static void mcl_base_args(hh_mcl* mc, hh_colargs& a) {
     a.stats = mc->d_stats;
     a.delta_bits = reinterpret_cast<int*>(mc->d_stats + 2);
     a.err = reinterpret_cast<int*>(mc->d_stats + 3);
-    a.flat = mc->flat > 0 ? 1 : 0;
-    a.l2pf = mc->l2pf > 0 ? 1 : 0;
 }
 
-// mean entries per (column, row block) segment below which the flat walk beats the segment-wise one
-// (measured on B200, 50k contigs: 32 -> segment-wise 180 ms vs flat 267 ms; 12 -> 71 ms vs 61 ms)
-static int choose_flat(const hh_mcl* mc, double nnz_operand) {
-    if (mc->flat >= 0) return mc->flat > 0;
+// Expansion inner loop by the mean entries per (column, row block) segment of the operand A: below 16 the flat walk beats
+// the segment-wise one (measured on B200, 50k contigs: 32 -> segment-wise 180 ms vs flat 267 ms; 12 -> 71 ms vs 61 ms).
+// The next batch's segments are prefetched into L2 in segment-wise mode only (long segments).
+static void choose_walk(const hh_mcl* mc, double nnz_operand, hh_colargs& a) {
     const double seg = nnz_operand / (double)mc->n / (double)mc->W;
-    return seg < 16.0 ? 1 : 0;
+    a.flat = seg < 16.0 ? 1 : 0;
+    a.l2pf = !a.flat;
 }
 
 // out[:, owned] = A . B[:, owned] as an unpruned slotted matrix: one factor of mkl_matrix_power's recursion
 // A . A^(k-1) (HapHiC_cluster.py:2017-2023) for --expansion k > 2
-static hh_geom mcl_geom(const hh_mcl* mc);
-static void mcl_base_args(hh_mcl* mc, hh_colargs& a);
-static int choose_flat(const hh_mcl* mc, double nnz_operand);
 static int raw_product(hh_mcl* mc, const hh_slotmat& A, const hh_slotmat& B, double nnz_a, hh_slotmat& out) {
     hh_colargs a;
     mcl_base_args(mc, a);
@@ -2427,8 +2295,7 @@ static int raw_product(hh_mcl* mc, const hh_slotmat& A, const hh_slotmat& B, dou
     a.B = B;
     a.out = out;
     a.raw = 1;
-    a.flat = choose_flat(mc, nnz_a);
-    a.l2pf = mc->l2pf >= 0 ? mc->l2pf : !a.flat;
+    choose_walk(mc, nnz_a, a);
     const hh_geom g = mcl_geom(mc);
     HH_CHECK((launch_col<SRC_PRODUCT, EPI_NORM>(mc->ctx, g, mc->d_scratch, mc->grid_cap, a)));
     return HH_OK;
@@ -2489,8 +2356,8 @@ extern "C" int hh_mcl_create_ex(hh_matrix* m, int expansion, int32_t col_lo, int
     mc->own_hi = col_hi;
     mc->expansion = expansion;
     mc->cur = -1;
-    mc->use_small = env_int("HH_MCL_SMALL", 1);
-    mc->use_window = env_int("HH_MCL_WINDOW", 1);
+    mc->use_small = 1;
+    mc->use_window = 1;
     mc->use_blk = env_int("HH_MCL_BLOCKGEMM", 1);
     if (expansion != 2) {          // higher powers go through the plain column kernel: A . (A . (... A)), one factor at a time
         mc->use_small = 0;
@@ -2498,8 +2365,6 @@ extern "C" int hh_mcl_create_ex(hh_matrix* m, int expansion, int32_t col_lo, int
         mc->use_blk = 0;
     }
     mc->blk_items = new std::vector<hh_gemm_item>();
-    mc->flat = env_int("HH_MCL_FLAT", -1);      // -1 = choose per launch from the mean segment length
-    mc->l2pf = env_int("HH_MCL_L2PF", -1);       // -1 = prefetch in segment-wise mode only (long segments)
     const hh_geom g = geom_for(ctx, m->n);
     mc->W = g.W;
     mc->T = g.T;
@@ -2602,9 +2467,8 @@ extern "C" int hh_mcl_create_ex(hh_matrix* m, int expansion, int32_t col_lo, int
         a.A = mc->m0;
         a.B = *Bp;
         a.dense_out = mc->d_m1;
-        a.flat = choose_flat(mc, (double)mc->nnz_m0);
-        const float pre_thr = (float)env_int("HH_MCL_PREORDER", 10);     // 0 = off; else link count that makes an edge "strong"
-        if (pre_thr > 0.f) {
+        choose_walk(mc, (double)mc->nnz_m0, a);
+        {   // column preorder: components of the strong-link graph
             const int n = m->n;
             int* d_lab = mc->d_comp_lo;        // n-sized scratch, rewritten by mcl_build_perm later
             int* d_flag = mc->d_bigcount + 2;
@@ -2613,7 +2477,7 @@ extern "C" int hh_mcl_create_ex(hh_matrix* m, int expansion, int32_t col_lo, int
             if (gridc > ctx->sm_count * 16) gridc = ctx->sm_count * 16;
             for (int round = 0; round < 64; ++round) {
                 HH_CUDA(cudaMemsetAsync(d_flag, 0, sizeof(int), ctx->stream));
-                HH_LAUNCH(ctx, hh_k_cc_hook_csc, gridc, 256, 0, m->d_colptr, m->d_row, m->d_val, n, pre_thr, d_lab, d_flag);
+                HH_LAUNCH(ctx, hh_k_cc_hook_csc, gridc, 256, 0, m->d_colptr, m->d_row, m->d_val, n, HH_PREORDER_STRONG, d_lab, d_flag);
                 HH_LAUNCH(ctx, hh_k_cc_jump, (n + 255) / 256, 256, 0, d_lab, n);
                 int changed = 0;
                 HH_CUDA(cudaMemcpyAsync(&changed, d_flag, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
@@ -2629,7 +2493,6 @@ extern "C" int hh_mcl_create_ex(hh_matrix* m, int expansion, int32_t col_lo, int
                 a.order = mc->d_order;
             }
         }
-        a.l2pf = mc->l2pf >= 0 ? mc->l2pf : !a.flat;
         if (expansion == 2) HH_CUDA(cudaEventRecord(mc->ev0, ctx->stream));
         HH_CHECK((launch_col<SRC_PRODUCT, EPI_DUMP>(ctx, g, mc->d_scratch, mc->grid_cap, a)));
         HH_CUDA(cudaEventRecord(mc->ev1, ctx->stream));
@@ -2709,7 +2572,6 @@ extern "C" int hh_mcl_fetch_m1(hh_mcl* mc, float* dense) {
 static int mcl_build_blk_items(hh_mcl* mc) {
     hh_ctx* ctx = mc->ctx;
     const int n = mc->n;
-    const int wlimit = env_int("HH_MCL_WMAX", 8192);
     mc->blk_items->clear();
     mc->blk_ldk = 0;
     mc->blk_flops = 0.0;
@@ -2723,7 +2585,7 @@ static int mcl_build_blk_items(hh_mcl* mc) {
         for (int p0 = 0; p0 < n;) {
             const int lo = clo[(size_t)p0], hi = chi[(size_t)p0];
             const int b = hi - lo;
-            if (b <= wlimit) {
+            if (b <= HH_WINDOW_MAX) {
                 if (b > maxb) maxb = b;
                 const int nt = (b + T - 1) / T, nkb = (b + 63) / 64;
                 for (int mt = 0; mt < nt; ++mt)
@@ -2783,7 +2645,6 @@ static int mcl_build_perm(hh_mcl* mc) {
         HH_LAUNCH(ctx, hh_k_cc_rank, (n + 255) / 256, 256, 0, d_lab, n, mc->d_perm, mc->d_inv, d_csize);
         HH_LAUNCH(ctx, hh_k_cc_ranges, (n + 255) / 256, 256, 0, d_lab, mc->d_perm, d_csize, n, mc->d_comp_lo, mc->d_comp_hi);
         // window size: the largest component that still fits (4 private accumulators of wmax floats, several CTAs per SM)
-        const int wlimit = env_int("HH_MCL_WMAX", 8192);
         if (!mc->h_inv) mc->h_inv = new std::vector<int>((size_t)n);
         HH_CUDA(cudaMemcpyAsync(mc->h_inv->data(), mc->d_inv, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
         std::vector<int> csz((size_t)n);
@@ -2791,27 +2652,13 @@ static int mcl_build_perm(hh_mcl* mc) {
         HH_CUDA(cudaStreamSynchronize(ctx->stream));
         int wmax = 32;
         for (int v = 0; v < n; ++v)
-            if (csz[(size_t)v] <= wlimit && csz[(size_t)v] > wmax) wmax = csz[(size_t)v];
-        if (env_int("HH_MCL_DEBUG", 0)) {
-            long long ncomp = 0, biggest = 0;
-            double cubes = 0.0;
-            for (int v = 0; v < n; ++v) {
-                const long long c = csz[(size_t)v];
-                if (c > 0) {
-                    ncomp++;
-                    cubes += (double)c * (double)c * (double)c;
-                    if (c > biggest) biggest = c;
-                }
-            }
-            fprintf(stderr, "[hh_mcl] inflation %.2f: iterate nnz %lld, %lld components, largest %lld, sum of cubes %.3e\n", (double)mc->inflation,
-                    (long long)mc->cur_nnz, ncomp, biggest, cubes);
-        }
+            if (csz[(size_t)v] <= HH_WINDOW_MAX && csz[(size_t)v] > wmax) wmax = csz[(size_t)v];
         mc->wmax = (wmax + 31) & ~31;
         // rewrite the iterate in new indices: column j' <- column inv[j'], rows through perm, rows re-sorted.
         // Columns of small components do it inside their window (one warp each); the others on the n-row accumulator.
         int all_counts[2] = {0, 0};
         HH_CUDA(cudaMemsetAsync(mc->d_bigcount, 0, 2 * sizeof(int), ctx->stream));
-        HH_LAUNCH(ctx, hh_k_cc_lists, (n + 255) / 256, 256, 0, mc->d_perm, 0, n, mc->d_comp_lo, mc->d_comp_hi, wlimit, mc->d_owned,
+        HH_LAUNCH(ctx, hh_k_cc_lists, (n + 255) / 256, 256, 0, mc->d_perm, 0, n, mc->d_comp_lo, mc->d_comp_hi, HH_WINDOW_MAX, mc->d_owned,
                   mc->d_win_list, mc->d_big_list, mc->d_bigcount);
         HH_CUDA(cudaMemcpyAsync(all_counts, mc->d_bigcount, 2 * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
         HH_CUDA(cudaMemsetAsync(mc->d_stats, 0, 4 * sizeof(unsigned long long), ctx->stream));
@@ -2846,7 +2693,7 @@ static int mcl_build_perm(hh_mcl* mc) {
         HH_REQUIRE((int)(st[3] & 0xffffffffull) == 0, HH_ERR_CAPACITY, "hh_mcl: slot overflow while relabelling");
         // the lists of the columns this context steps
         HH_CUDA(cudaMemsetAsync(mc->d_bigcount, 0, 2 * sizeof(int), ctx->stream));
-        HH_LAUNCH(ctx, hh_k_cc_lists, (ncols + 255) / 256, 256, 0, mc->d_perm, mc->col_lo, ncols, mc->d_comp_lo, mc->d_comp_hi, wlimit,
+        HH_LAUNCH(ctx, hh_k_cc_lists, (ncols + 255) / 256, 256, 0, mc->d_perm, mc->col_lo, ncols, mc->d_comp_lo, mc->d_comp_hi, HH_WINDOW_MAX,
                   mc->d_owned, mc->d_win_list, mc->d_big_list, mc->d_bigcount);
         int counts[2] = {0, 0};
         HH_CUDA(cudaMemcpyAsync(counts, mc->d_bigcount, 2 * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
@@ -2883,11 +2730,9 @@ extern "C" int hh_mcl_begin(hh_mcl* mc, double inflation, double pruning) {
     mc->inflation = (float)inflation;
     mc->inflate_square = HH_INFL_POW;                 // how x^r is evaluated (hh_inflate)
     if (mc->inflation == 2.0f) mc->inflate_square = HH_INFL_SQUARE;
-    else if (env_int("HH_MCL_FAST_POW", 1)) {
-        if (mc->inflation == 1.5f) mc->inflate_square = HH_INFL_X15;
-        else if (mc->inflation == 3.0f) mc->inflate_square = HH_INFL_CUBE;
-        else if (mc->inflation == 2.5f) mc->inflate_square = HH_INFL_X25;
-    }
+    else if (mc->inflation == 1.5f) mc->inflate_square = HH_INFL_X15;
+    else if (mc->inflation == 3.0f) mc->inflate_square = HH_INFL_CUBE;
+    else if (mc->inflation == 2.5f) mc->inflate_square = HH_INFL_X25;
     mc->prune = (float)pruning;   // `matrix >= pruning` compares in fp32
     mc->cur = -1;
     mc->have_pending = false;
@@ -2923,13 +2768,7 @@ extern "C" int hh_mcl_step(hh_mcl* mc, int it, int64_t* nnz_owned, int64_t* prod
     if (it == 0) {
         a.dense_in = mc->d_m1;
         a.do_conv = 0;
-        if (mc->perm_space) {              // new indices: source column inv[j'], rows scattered through perm
-            a.perm = mc->d_perm;
-            a.orig = mc->d_inv;
-            a.order = mc->d_owned;
-        }
-        if (!mc->perm_space && env_int("HH_MCL_ITER0_STREAM", 1)) HH_CHECK(launch_iter0(ctx, g, a));
-        else HH_CHECK((launch_col<SRC_DENSE, EPI_PRUNE>(ctx, g, mc->d_scratch, mc->grid_cap, a)));
+        HH_CHECK(launch_iter0(ctx, g, a));      // original indices: the relabelling is built after iteration 0
     } else if (mc->perm_space) {
         a.A = mc->it[mc->cur];
         a.B = mc->it[mc->cur];
@@ -2937,8 +2776,7 @@ extern "C" int hh_mcl_step(hh_mcl* mc, int it, int64_t* nnz_owned, int64_t* prod
         a.orig = mc->d_inv;
         const double dcol = (double)mc->cur_nnz / (double)mc->n;
         a.track = (dcol * dcol * 4.0 < (double)mc->n) ? 1 : 0;
-        a.flat = choose_flat(mc, (double)mc->cur_nnz);
-        a.l2pf = mc->l2pf >= 0 ? mc->l2pf : !a.flat;
+        choose_walk(mc, (double)mc->cur_nnz, a);
         a.T = g.T;
         if (mc->use_small && mc->cur_nnz <= 8ll * mc->n) {
             HH_CUDA(cudaMemsetAsync(mc->d_bigcount, 0, sizeof(int), ctx->stream));
@@ -2987,7 +2825,7 @@ extern "C" int hh_mcl_step(hh_mcl* mc, int it, int64_t* nnz_owned, int64_t* prod
                 hh_gemm_operand B = {d_blkB, np_op, mc->n, (int)mc->blk_ldk, mc->blk_ldk, (long long)plane, fmt};
                 HH_CHECK(hh_gemm_run(ctx, A, B, mc->d_blk_items, (int)mc->blk_items->size(), npass, pa, pb,
                                      env_int("HH_GEMM_CHUNK", f16 ? 2 : 1), d_blk_out, mc->blk_ldk, 0, mc->n, nullptr, nullptr,
-                                     hh_gemm_blk_out_scale(f16), 0, 0));
+                                     hh_gemm_blk_out_scale(f16), 0));
                 a.dense_in = d_blk_out;
                 a.ld = mc->blk_ldk;
                 mc->blk_iters++;
@@ -3032,8 +2870,7 @@ extern "C" int hh_mcl_step(hh_mcl* mc, int it, int64_t* nnz_owned, int64_t* prod
         // expected products per column ~ (nnz/n)^2; track dirty chunks when that is well below n
         const double dcol = (double)mc->cur_nnz / (double)mc->n;
         a.track = (dcol * dcol * 4.0 < (double)mc->n) ? 1 : 0;
-        a.flat = choose_flat(mc, (double)mc->cur_nnz);
-        a.l2pf = mc->l2pf >= 0 ? mc->l2pf : !a.flat;
+        choose_walk(mc, (double)mc->cur_nnz, a);
         if (mc->use_small && mc->cur_nnz <= 8ll * mc->n) {
             // nearly converged: one warp per column; what does not fit goes to the accumulator kernel
             const int ncols = mc->col_hi - mc->col_lo;
@@ -3136,9 +2973,8 @@ extern "C" int hh_mcl_set_block(hh_mcl* mc, int32_t col_lo, int32_t col_hi) {
     mc->col_hi = col_hi;
     if (mc->perm_space) {
         const int ncols = col_hi - col_lo;
-        const int wlimit = env_int("HH_MCL_WMAX", 8192);
         HH_CUDA(cudaMemsetAsync(mc->d_bigcount, 0, 2 * sizeof(int), ctx->stream));
-        HH_LAUNCH(ctx, hh_k_cc_lists, (ncols + 255) / 256, 256, 0, mc->d_perm, mc->col_lo, ncols, mc->d_comp_lo, mc->d_comp_hi, wlimit,
+        HH_LAUNCH(ctx, hh_k_cc_lists, (ncols + 255) / 256, 256, 0, mc->d_perm, mc->col_lo, ncols, mc->d_comp_lo, mc->d_comp_hi, HH_WINDOW_MAX,
                   mc->d_owned, mc->d_win_list, mc->d_big_list, mc->d_bigcount);
         int counts[2] = {0, 0};
         HH_CUDA(cudaMemcpyAsync(counts, mc->d_bigcount, 2 * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));

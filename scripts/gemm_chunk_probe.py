@@ -1,6 +1,6 @@
 """Pre-expansion GEMM at C3 under different drain periods / encodings (env switches of csrc/hh_gemm.cu): one link matrix,
 one `Mcl(...)` per variant, prints the engine's own timings.  Usage: python scripts/gemm_chunk_probe.py [variant ...] with
-variant = FMT:CHUNK[:SPLIT] (e.g. f16:6:1 f16:8:0 bf16:2)."""
+variant = FMT:CHUNK (e.g. f16:3 f16:8 bf16:2)."""
 import json
 import os
 import sys
@@ -12,7 +12,7 @@ from haphic_b200._lib import Context
 from haphic_b200.links import LinkTable, name_rank
 from haphic_b200.mcl import Mcl
 
-variants = sys.argv[1:] or ["f16:4:1", "f16:6:1", "f16:8:1", "f16:12:1", "f16:8:0", "f16:3:0", "bf16:2"]
+variants = sys.argv[1:] or ["f16:3", "f16:4", "f16:6", "f16:8", "f16:12", "bf16:2"]
 pairs = int(os.environ.get("PAIRS", "200000000"))
 asm = synth.make_assembly(24, 50000, 20000, seed=12345)
 rank = name_rank(asm.names)
@@ -29,10 +29,9 @@ mat = tab.to_matrix(keep, np.nonzero(index < 0)[0].astype(np.int32))
 NC = 512                                    # columns of the accuracy check: exact fp64 product of the fp32 M0
 exact = None
 for v in variants:
-    fmt, chunk, split = (v.split(":") + ["1"])[:3]
+    fmt, chunk = v.split(":")
     os.environ["HH_GEMM_FMT"] = fmt
     os.environ["HH_GEMM_CHUNK"] = chunk
-    os.environ["HH_GEMM_SPLIT"] = split
     mc = Mcl(mat, preexp="dense")
     mc2 = Mcl(mat, preexp="dense")          # second construction: warm allocator
     p = mc2.preexp

@@ -1,6 +1,5 @@
-"""Iteration 0 (hh_k_iter0: stream of the dense pre-expanded matrix) at C3 for the CTA shapes HH_MCL_IT0_WARPS = 8 / 16 / 32:
-device time of the kernel and the number of surviving entries (must not depend on the shape); `queue` = the variant that
-collects the candidates of passes 2 and 3 in a per-warp queue first."""
+"""Iteration 0 (hh_k_iter0: stream of the dense pre-expanded matrix) at C3: device time of the kernel and the number of
+surviving entries per inflation."""
 import json
 import os
 import sys
@@ -24,16 +23,12 @@ keep = np.ones(asm.n, np.uint8)
 index, _ = tab.linked_index(keep)
 mat = tab.to_matrix(keep, np.nonzero(index < 0)[0].astype(np.int32))
 mc = Mcl(mat, preexp="dense")
-for nw in (sys.argv[1:] or ["queue", "8", "16", "32"]):
-    # "queue": candidates of passes 2 and 3 evaluated 32 at a time (8-warp CTAs); a number: the direct evaluation with that shape
-    os.environ["HH_MCL_IT0_QUEUE"] = "1" if nw == "queue" else "0"
-    os.environ["HH_MCL_IT0_WARPS"] = "8" if nw == "queue" else nw
-    out = {"variant": nw}
-    for r in (2.0, 1.5, 3.0, 1.7):
-        best, nnz = 1e9, None
-        for _ in range(3):
-            st = mc.run(r, 1, 1e-4)
-            best = min(best, float(st["iter_ms"][0]))
-            nnz = int(st["iter_nnz"][0])
-        out["r{}".format(r)] = {"ms": round(best, 3), "nnz": nnz}
-    print("IT0 " + json.dumps(out), flush=True)
+out = {}
+for r in (2.0, 1.5, 3.0, 1.7):
+    best, nnz = 1e9, None
+    for _ in range(3):
+        st = mc.run(r, 1, 1e-4)
+        best = min(best, float(st["iter_ms"][0]))
+        nnz = int(st["iter_nnz"][0])
+    out["r{}".format(r)] = {"ms": round(best, 3), "nnz": nnz}
+print("IT0 " + json.dumps(out), flush=True)
