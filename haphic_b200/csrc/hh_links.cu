@@ -279,7 +279,7 @@ hh_k_links_insert(const int4* __restrict__ rec, int64_t n_rec, uint32_t stream_o
 // records are therefore first split by the high bits of the key hash into 2^npart_log partitions (one sequential read,
 // one write in runs that fill whole sectors).  A partition is still far too large for shared memory, and counting the
 // partitions one launch at a time in an L2-resident table is a chain of latency-bound launches, so every partition is
-// split again by the next hash bits into sub-partitions of at most ~1k records, and ONE launch counts all of them, a
+// split again by the next hash bits into sub-partitions of at most 512 records, and ONE launch counts all of them, a
 // CTA per sub-partition in a shared-memory table, emitting compact entries (9 words, the hh_links_adopt list format).
 // Integer adds and mins only: the result is identical to the direct path.
 //   hh_k_part_scatter   record -> {i, j, stream index, flags} (ends ordered by name rank, is_flank / head-tail evaluated once)
@@ -292,6 +292,9 @@ hh_k_links_insert(const int4* __restrict__ rec, int64_t n_rec, uint32_t stream_o
 #define HH_PART_TILE 4096          // records per tile of the scatter kernel (512 threads x 8)
 #define HH_PART_MAX 1024
 
+// The tile kernels below work in phases: the 8 record loads of a thread are issued together, then the lookups that depend
+// on them, then the shared-memory atomics.  Written as one loop per record, the compiler keeps each record's load behind
+// the previous record's atomic, and a tile waits through eight DRAM latencies one after the other.
 __global__ void __launch_bounds__(512)
 hh_k_part_scatter(const int4* __restrict__ rec, int64_t n_rec, uint32_t stream_off, int32_t n_ctg, const int32_t* __restrict__ ctg_len,
                   const int32_t* __restrict__ name_rank, const uint8_t* __restrict__ in_nx, int64_t flank_bp, int npart_log,
@@ -306,37 +309,41 @@ hh_k_part_scatter(const int4* __restrict__ rec, int64_t n_rec, uint32_t stream_o
     if (threadIdx.x == 0) s_used = 0;
     for (int64_t t = blockIdx.x; t < tiles; t += gridDim.x) {
         for (int k = threadIdx.x; k < npart; k += 512) s_cnt[k] = 0;
-        __syncthreads();
         int4 out[8];
         int part[8];
         unsigned int rnk[8];
 #pragma unroll
         for (int k = 0; k < 8; ++k) {
             const int64_t i = t * HH_PART_TILE + (int64_t)k * 512 + threadIdx.x;
+            out[k] = (i < n_rec) ? hh_ld_stream(rec + i) : make_int4(-1, 0, -1, 0);
+        }
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+            int a = out[k].x, b = out[k].z, pa = out[k].y, pb = out[k].w;
             part[k] = -1;
-            if (i < n_rec) {
-                const int4 r = hh_ld_stream(rec + i);
-                int a = r.x, b = r.z, pa = r.y, pb = r.w;
-                if (a != b && (unsigned)a < (unsigned)n_ctg && (unsigned)b < (unsigned)n_ctg) {
-                    if (name_rank[a] > name_rank[b]) {      // sorted(((ref,pos+1),(mref,mpos+1))), 1629
-                        int x = a; a = b; b = x;
-                        x = pa; pa = pb; pb = x;
-                    }
-                    const int64_t coord_i = (int64_t)pa + 1, coord_j = (int64_t)pb + 1;
-                    const int64_t li = ctg_len[a], lj = ctg_len[b];
-                    const bool fi = (flank_bp == 0) || (coord_i <= flank_bp) || (coord_i > li - flank_bp);   // is_flank, 299-307
-                    const bool fj = (flank_bp == 0) || (coord_j <= flank_bp) || (coord_j > lj - flank_bp);
-                    const unsigned fl = (fi && fj && in_nx[a] && in_nx[b]) ? 1u : 0u;                         // 1636
-                    const unsigned ti = (coord_i * 2 > li) ? 2u : 0u, tj = (coord_j * 2 > lj) ? 4u : 0u;       // 404-416
-                    const uint64_t key = ((uint64_t)(uint32_t)a << 32) | (uint64_t)(uint32_t)b;
-                    const int p = (int)(hh_mix64(key) >> (64 - npart_log));
-                    part[k] = p;
-                    rnk[k] = atomicAdd(&s_cnt[p], 1u);
-                    out[k] = make_int4(a, b, (int)(stream_off + (uint32_t)i), (int)(fl | ti | tj | ((unsigned)p << 8)));
-                    my_used++;
+            if (a != b && (unsigned)a < (unsigned)n_ctg && (unsigned)b < (unsigned)n_ctg) {
+                if (name_rank[a] > name_rank[b]) {      // sorted(((ref,pos+1),(mref,mpos+1))), 1629
+                    int x = a; a = b; b = x;
+                    x = pa; pa = pb; pb = x;
                 }
+                const int64_t coord_i = (int64_t)pa + 1, coord_j = (int64_t)pb + 1;
+                const int64_t li = ctg_len[a], lj = ctg_len[b];
+                const bool fi = (flank_bp == 0) || (coord_i <= flank_bp) || (coord_i > li - flank_bp);   // is_flank, 299-307
+                const bool fj = (flank_bp == 0) || (coord_j <= flank_bp) || (coord_j > lj - flank_bp);
+                const unsigned fl = (fi && fj && in_nx[a] && in_nx[b]) ? 1u : 0u;                         // 1636
+                const unsigned ti = (coord_i * 2 > li) ? 2u : 0u, tj = (coord_j * 2 > lj) ? 4u : 0u;       // 404-416
+                const uint64_t key = ((uint64_t)(uint32_t)a << 32) | (uint64_t)(uint32_t)b;
+                const int p = (int)(hh_mix64(key) >> (64 - npart_log));
+                const int64_t i = t * HH_PART_TILE + (int64_t)k * 512 + threadIdx.x;
+                part[k] = p;
+                out[k] = make_int4(a, b, (int)(stream_off + (uint32_t)i), (int)(fl | ti | tj | ((unsigned)p << 8)));
+                my_used++;
             }
         }
+        __syncthreads();
+#pragma unroll
+        for (int k = 0; k < 8; ++k)
+            if (part[k] >= 0) rnk[k] = atomicAdd(&s_cnt[part[k]], 1u);
         __syncthreads();
         for (int k = threadIdx.x; k < npart; k += 512)
             if (s_cnt[k]) s_base[k] = atomicAdd(cursor + k, (unsigned long long)s_cnt[k]);
@@ -363,8 +370,13 @@ hh_k_part_scatter(const int4* __restrict__ rec, int64_t n_rec, uint32_t stream_o
 }
 
 #define HH_SUB_MAX_LOG 10          // at most 2^10 sub-partitions per partition
-#define HH_SUB_SLOTS 2048          // slots of the shared-memory table: a sub-partition is sized for <= HH_SUB_SLOTS / 2 records
-#define HH_SUB_SMEM (HH_SUB_SLOTS * 36)   // u64 key + 7 u32 counters a slot: 72 KB, three CTAs an SM
+// Slots of the shared-memory table: a sub-partition is sized for <= HH_SUB_SLOTS / 2 records.  Measured at C3 on a B200, the
+// count runs faster the more warps an SM holds: 2048 slots (two CTAs an SM with the record buffers) 10.9 ms, 1024 slots
+// (four CTAs) 7.4 ms.
+#define HH_SUB_SLOTS 1024
+#define HH_SUB_CHUNK (HH_SUB_SLOTS / 2)   // records a record buffer of hh_k_sub_count holds
+// two record buffers of 16 B records, u64 key + 7 u32 counters a slot, u16 live-slot list: 54 KB, four CTAs an SM
+#define HH_SUB_SMEM (2 * HH_SUB_CHUNK * 16 + HH_SUB_SLOTS * (36 + 2))
 
 __device__ __forceinline__ unsigned hh_sub_of(const int4 r, int npart_log, int sub_log) {
     const uint64_t key = ((uint64_t)(uint32_t)r.x << 32) | (uint64_t)(uint32_t)r.y;
@@ -405,16 +417,22 @@ hh_k_sub_split(const int4* __restrict__ pbuf, uint64_t pcap, const unsigned long
         int4 r[8];
         int s[8];
         unsigned int rnk[8];
+        // phases as in hh_k_part_scatter: all loads, then the sub-partition ids, then the atomics
 #pragma unroll
         for (int k = 0; k < 8; ++k) {
             const int64_t i = t * HH_PART_TILE + (int64_t)k * 512 + threadIdx.x;
-            s[k] = -1;
-            if (i < n) {
-                r[k] = hh_ld_stream(src + i);
-                s[k] = (int)hh_sub_of(r[k], npart_log, sub_log);
-                if (SCATTER) rnk[k] = atomicAdd(&s_cnt[s[k]], 1u);
-                else atomicAdd(&s_cnt[s[k]], 1u);
-            }
+            if (i < n) r[k] = hh_ld_stream(src + i);
+        }
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+            const int64_t i = t * HH_PART_TILE + (int64_t)k * 512 + threadIdx.x;
+            s[k] = (i < n) ? (int)hh_sub_of(r[k], npart_log, sub_log) : -1;
+        }
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+            if (s[k] < 0) continue;
+            if (SCATTER) rnk[k] = atomicAdd(&s_cnt[s[k]], 1u);
+            else atomicAdd(&s_cnt[s[k]], 1u);
         }
         if (SCATTER) {
             __syncthreads();
@@ -471,17 +489,29 @@ hh_k_sub_offsets(unsigned int* __restrict__ sub_cnt, int sub_log, const int64_t*
     if (blockIdx.x == npart - 1 && threadIdx.x == 0) sub_off[(size_t)npart << sub_log] = pbase[npart];
 }
 
+// 16-byte asynchronous global -> shared copies (bypassing L1), in commit groups
+__device__ __forceinline__ void hh_cp_async16(void* smem, const void* gmem) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem)), "l"(gmem) : "memory");
+}
+__device__ __forceinline__ void hh_cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+__device__ __forceinline__ void hh_cp_async_wait_prev() { asm volatile("cp.async.wait_group 1;" ::: "memory"); }
+
 // Count + emit: a CTA takes sub-partitions in a grid stride, counts each into an open-addressing table in shared memory
-// (warp aggregation with match.any as in hh_part_count, then shared-memory atomics), and emits the live slots with a block
-// scan and ONE global atomic on the entry cursor.  Nothing global is touched before the emit.  A sub-partition whose keys do
-// not fit the table (skewed or adversarial keys only) is abandoned and its id appended to `fallback` (counters[7] entries)
-// for the global scratch-table path (hh_k_part_step).
+// (warp aggregation with match.any as in hh_part_count, then shared-memory atomics), and emits the slots it filled with ONE
+// global atomic on the entry cursor.  Nothing global is touched before the emit.  A sub-partition whose keys do not fit the
+// table (skewed or adversarial keys only) is abandoned and its id appended to `fallback` (counters[7] entries) for the
+// global scratch-table path (hh_k_part_step).
+// The records come in chunks of HH_SUB_CHUNK (a whole sub-partition, unless it is a hot one), copied into one of two
+// shared-memory buffers while the chunk before is counted from the other.  Every slot a CTA inserts is appended to a list of
+// live slots: the emit walks that list (its index is the entry's output position) and resets only those slots, so the table
+// is cleared once, at kernel start.
 __global__ void __launch_bounds__(256)
 hh_k_sub_count(const int4* __restrict__ prec, const int64_t* __restrict__ sub_off, int nsub_total, uint32_t* __restrict__ compact,
                uint64_t compact_cap, unsigned long long* __restrict__ ctg_links, unsigned long long* __restrict__ counters,
                uint32_t* __restrict__ fallback) {
-    constexpr int S = HH_SUB_SLOTS, E = HH_SUB_SLOTS / 256;
-    extern __shared__ uint64_t s_keys[];                   // [S], then 7 x u32 [S]
+    constexpr int S = HH_SUB_SLOTS, C = HH_SUB_CHUNK;
+    extern __shared__ int4 s_rec[];                        // [2][C] records, then u64 keys [S], 7 x u32 [S], u16 live [S]
+    uint64_t* s_keys = reinterpret_cast<uint64_t*>(s_rec + 2 * C);
     uint32_t* s_ff = reinterpret_cast<uint32_t*>(s_keys + S);
     uint32_t* s_ffl = s_ff + S;
     uint32_t* s_full = s_ffl + S;
@@ -489,30 +519,60 @@ hh_k_sub_count(const int4* __restrict__ prec, const int64_t* __restrict__ sub_of
     uint32_t* s_ht = s_fl + S;
     uint32_t* s_th = s_ht + S;
     uint32_t* s_tt = s_th + S;
-    __shared__ unsigned int s_over, s_wtot[8];
+    uint16_t* s_live = reinterpret_cast<uint16_t*>(s_tt + S);
+    __shared__ unsigned int s_over, s_nlive;
     __shared__ unsigned long long s_base;
     const int lane = threadIdx.x & 31, wv = threadIdx.x >> 5;
     unsigned int nfl = 0;
-    for (int id = blockIdx.x; id < nsub_total; id += gridDim.x) {
-        for (int k = threadIdx.x; k < S; k += 256) {
-            s_keys[k] = HH_EMPTY_KEY;
-            s_ff[k] = HH_NONE32;
-            s_ffl[k] = HH_NONE32;
-            s_full[k] = 0u;
-            s_fl[k] = 0u;
-            s_ht[k] = 0u;
-            s_th[k] = 0u;
-            s_tt[k] = 0u;
+    for (int k = threadIdx.x; k < S; k += 256) {
+        s_keys[k] = HH_EMPTY_KEY;
+        s_ff[k] = HH_NONE32;
+        s_ffl[k] = HH_NONE32;
+        s_full[k] = 0u;
+        s_fl[k] = 0u;
+        s_ht[k] = 0u;
+        s_th[k] = 0u;
+        s_tt[k] = 0u;
+    }
+    if (threadIdx.x == 0) {
+        s_over = 0u;
+        s_nlive = 0u;
+    }
+    // the chunk being counted (sub-partition id, records [b + off, b + off + C) of its n) and the bounds of the CTA's next
+    // sub-partition, loaded one sub-partition ahead
+    int id = blockIdx.x;
+    int64_t off = 0, b = 0, n = 0, nb = 0, nn = 0;
+    if (id < nsub_total) {
+        b = sub_off[id];
+        n = sub_off[id + 1] - b;
+        for (int k = threadIdx.x; k < (int)min(n, (int64_t)C); k += 256) hh_cp_async16(s_rec + k, prec + b + k);
+    }
+    hh_cp_async_commit();
+    if (id + (int)gridDim.x < nsub_total) {
+        nb = sub_off[id + gridDim.x];
+        nn = sub_off[id + gridDim.x + 1] - nb;
+    }
+    int buf = 0;
+    while (id < nsub_total) {
+        // start the copy of the next chunk: the rest of this sub-partition, or the first chunk of the next one
+        const bool last = off + C >= n;
+        {
+            const int64_t src = last ? nb : b + off + C;
+            const int m = (int)min(last ? nn : n - off - C, (int64_t)C);
+            if (!last || id + (int)gridDim.x < nsub_total)
+                for (int k = threadIdx.x; k < m; k += 256) hh_cp_async16(s_rec + (buf ^ 1) * C + k, prec + src + k);
+            hh_cp_async_commit();
         }
-        if (threadIdx.x == 0) s_over = 0u;
-        __syncthreads();
-        const int64_t b = sub_off[id], n = sub_off[id + 1] - b;
-        for (int64_t i0 = (int64_t)wv * 32; i0 < n; i0 += 256) {
+        hh_cp_async_wait_prev();
+        __syncthreads();                       // the chunk is in shared memory, the table reset of the last emit is done
+        const int4* rc = s_rec + buf * C;
+        const int m = (int)min(n - off, (int64_t)C);
+        for (int i0 = wv * 32; i0 < m; i0 += 256) {
             if (__any_sync(HH_FULL_MASK, *(volatile unsigned int*)&s_over != 0u)) break;
-            const int64_t i = i0 + lane;
-            const bool ok = i < n;
+            const int i = i0 + lane;
+            const bool ok = i < m;
             int4 r = make_int4(0, 0, 0, 0);
-            if (ok) r = hh_ld_stream(prec + b + i);
+            if (ok) r = rc[i];
             const unsigned f = (unsigned)r.w;
             const uint64_t key = ok ? (((uint64_t)(uint32_t)r.x << 32) | (uint64_t)(uint32_t)r.y) : (HH_EMPTY_KEY - 1 - (uint64_t)lane);
             const unsigned peers = __match_any_sync(HH_FULL_MASK, key);
@@ -533,6 +593,7 @@ hh_k_sub_count(const int4* __restrict__ prec, const int64_t* __restrict__ sub_of
                     if (k == HH_EMPTY_KEY) {
                         const unsigned long long prev = atomicCAS((unsigned long long*)(s_keys + sl), (unsigned long long)HH_EMPTY_KEY,
                                                                   (unsigned long long)key);
+                        if (prev == HH_EMPTY_KEY) s_live[atomicAdd(&s_nlive, 1u)] = (uint16_t)sl;
                         if (prev == HH_EMPTY_KEY || prev == key) { found = true; break; }
                     }
                     sl = (sl + 1) & (S - 1);
@@ -554,62 +615,67 @@ hh_k_sub_count(const int4* __restrict__ prec, const int64_t* __restrict__ sub_of
                 }
             }
         }
-        __syncthreads();
-        if (s_over) {
-            if (threadIdx.x == 0) fallback[atomicAdd(counters + 7, 1ull)] = (uint32_t)id;
-            __syncthreads();                   // s_over is read by every thread before the next sub-partition resets it
-            continue;
-        }
-        // ---- emit: live slots -> compact entries {i, j, full, flank, first_full, first_flank, HT, TH, TT}, per-fragment totals
-        unsigned int cnt = 0;
-#pragma unroll
-        for (int q = 0; q < E; ++q) cnt += (s_keys[q * 256 + threadIdx.x] != HH_EMPTY_KEY) ? 1u : 0u;
-        unsigned int incl = cnt;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const unsigned int t = __shfl_up_sync(HH_FULL_MASK, incl, o);
-            if (lane >= o) incl += t;
-        }
-        if (lane == 31) s_wtot[wv] = incl;
-        __syncthreads();
-        unsigned int before = 0, total = 0;
-#pragma unroll
-        for (int k = 0; k < 8; ++k) {
-            const unsigned int t = s_wtot[k];
-            before += (k < wv) ? t : 0u;
-            total += t;
-        }
-        if (threadIdx.x == 0) s_base = total ? atomicAdd(counters + 0, (unsigned long long)total) : 0ull;
-        __syncthreads();
-        unsigned long long pos = s_base + before + (incl - cnt);
-#pragma unroll
-        for (int q = 0; q < E; ++q) {
-            const int sl = q * 256 + threadIdx.x;
-            const uint64_t key = s_keys[sl];
-            if (key == HH_EMPTY_KEY) continue;
-            const uint32_t flank = s_fl[sl];
-            if (pos < compact_cap) {
-                uint32_t* o = compact + pos * 9;
-                o[0] = (uint32_t)(key >> 32);
-                o[1] = (uint32_t)key;
-                o[2] = s_full[sl];
-                o[3] = flank;
-                o[4] = s_ff[sl];
-                o[5] = s_ffl[sl];
-                o[6] = s_ht[sl];
-                o[7] = s_th[sl];
-                o[8] = s_tt[sl];
-            } else {
-                atomicExch(counters + 2, 5ull);
+        __syncthreads();                       // every warp is done with this chunk's buffer and its table updates
+        if (last) {
+            // ---- emit: live slots -> compact entries {i, j, full, flank, first_full, first_flank, HT, TH, TT}, per-fragment
+            // totals; every live slot is reset for the next sub-partition
+            const unsigned int nl = s_nlive;
+            const bool over = s_over != 0u;
+            __syncthreads();
+            if (threadIdx.x == 0) {
+                s_base = (!over && nl) ? atomicAdd(counters + 0, (unsigned long long)nl) : 0ull;
+                if (over) fallback[atomicAdd(counters + 7, 1ull)] = (uint32_t)id;
+                s_nlive = 0u;
+                s_over = 0u;
             }
-            pos++;
-            if (flank) {
-                nfl++;
-                atomicAdd(ctg_links + (uint32_t)(key >> 32), (unsigned long long)flank);      // ctg_link_dict (1638-1639)
-                atomicAdd(ctg_links + (uint32_t)key, (unsigned long long)flank);
+            __syncthreads();
+            for (unsigned int t = threadIdx.x; t < nl; t += 256) {
+                const int sl = s_live[t];
+                if (!over) {
+                    const uint64_t key = s_keys[sl];
+                    const uint32_t flank = s_fl[sl];
+                    const unsigned long long pos = s_base + t;
+                    if (pos < compact_cap) {
+                        uint32_t* o = compact + pos * 9;
+                        o[0] = (uint32_t)(key >> 32);
+                        o[1] = (uint32_t)key;
+                        o[2] = s_full[sl];
+                        o[3] = flank;
+                        o[4] = s_ff[sl];
+                        o[5] = s_ffl[sl];
+                        o[6] = s_ht[sl];
+                        o[7] = s_th[sl];
+                        o[8] = s_tt[sl];
+                    } else {
+                        atomicExch(counters + 2, 5ull);
+                    }
+                    if (flank) {
+                        nfl++;
+                        atomicAdd(ctg_links + (uint32_t)(key >> 32), (unsigned long long)flank);      // ctg_link_dict (1638-1639)
+                        atomicAdd(ctg_links + (uint32_t)key, (unsigned long long)flank);
+                    }
+                }
+                s_keys[sl] = HH_EMPTY_KEY;
+                s_ff[sl] = HH_NONE32;
+                s_ffl[sl] = HH_NONE32;
+                s_full[sl] = 0u;
+                s_fl[sl] = 0u;
+                s_ht[sl] = 0u;
+                s_th[sl] = 0u;
+                s_tt[sl] = 0u;
             }
+            id += gridDim.x;
+            off = 0;
+            b = nb;
+            n = nn;
+            if (id + (int)gridDim.x < nsub_total) {
+                nb = sub_off[id + gridDim.x];
+                nn = sub_off[id + gridDim.x + 1] - nb;
+            }
+        } else {
+            off += C;
         }
-        __syncthreads();                       // the table and s_wtot / s_base are reused by the next sub-partition
+        buf ^= 1;
     }
     nfl = (unsigned)hh_warp_sum((int)nfl);
     if (lane == 0 && nfl) atomicAdd(counters + 3, (unsigned long long)nfl);
@@ -1275,9 +1341,11 @@ static int links_launch_insert(hh_links* lk, const int4* d_rec, int64_t n_rec, i
                                const uint32_t* d_pos = nullptr) {
     hh_ctx* ctx = lk->ctx;
     if (lk->mode == 2 && d_pos == nullptr) {
+        // one wave of resident CTAs, each taking tiles in a grid stride
         const int64_t tiles = (n_rec + HH_PART_TILE - 1) / HH_PART_TILE;
-        int grid = (int)(tiles < (int64_t)hh_grid(ctx, 3) ? tiles : (int64_t)hh_grid(ctx, 3));
-        if (grid < 1) grid = 1;
+        int per_sm = 0;
+        HH_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, hh_k_part_scatter, 512, 0));
+        const int grid = (int)std::max<int64_t>(1, std::min(tiles, (int64_t)hh_grid(ctx, std::max(per_sm, 1))));
         const hh_partset& ps = lk->psets->back();
         HH_LAUNCH(ctx, hh_k_part_scatter, grid, 512, 0, d_rec, n_rec, (uint32_t)stream_offset, lk->n_ctg, lk->d_len, lk->d_rank, lk->d_nx,
                   lk->flank_bp, lk->npart_log, ps.buf, ps.pcap, ps.cursor, lk->d_spill, lk->spill_cap, lk->d_spill_cursor,
