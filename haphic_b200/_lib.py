@@ -102,6 +102,18 @@ _SIGNATURES = {
     "hh_bam_close": (C.c_int, [_P]),
     "hh_pickle_links": (C.c_int, [C.c_char_p, _P, C.c_int32, _P, _P, C.c_int64, _P, _P, _P]),
     "hh_clm_from_records": (C.c_int, [C.c_char_p, _P, C.c_int32, _P, C.c_int64, _P, _P, C.c_int]),
+    "hh_correct_create": (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.POINTER(_P)]),
+    "hh_correct_add": (C.c_int, [_P, _P, C.c_int64, C.c_int]),
+    "hh_correct_info": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "hh_correct_fetch": (C.c_int, [_P, _P, _P, _P]),
+    "hh_correct_detect": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_double, C.c_double, C.c_int64, _P, _P, _P, C.c_int64,
+                                    C.POINTER(C.c_int64)]),
+    "hh_correct_detect_segments": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, _P, _P, _P, C.c_double, C.c_double,
+                                             C.c_int64, _P, _P, _P, C.c_int64, C.POINTER(C.c_int64)]),
+    "hh_correct_split": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_int32]),
+    "hh_correct_set_pieces": (C.c_int, [_P, C.c_int32, _P, _P, _P]),
+    "hh_correct_remap": (C.c_int, [_P, _P, C.c_int64, C.c_int]),
+    "hh_correct_destroy": (C.c_int, [_P]),
 }
 
 _lib = None

@@ -10,8 +10,9 @@ unchanged.  The per-read-pair link counting, dict_to_matrix and the Markov-clust
 libhaphic_b200.so on the GPU; file parsing, fragment statistics, filters on per-fragment scalars,
 result interpretation and the writers are host Python, as in the reference.
 
-Not supported (raise, never silently degrade): ``--correct_nrounds``, ``--ul``, ``--gfa`` (out of the hot-path scope,
-SURVEY.md section 2).
+``--correct_nrounds`` (assembly correction, 943-1297) runs on the GPU as well (haphic_b200/correct.py, hh_correct.cu).
+
+Not supported (raise, never silently degrade): ``--ul``, ``--gfa`` (out of the hot-path scope, SURVEY.md section 2).
 
 Reference line numbers below refer to scripts/HapHiC_cluster.py (v1.0.7).
 """
@@ -1271,7 +1272,10 @@ def run(args, log_file=None):
                     "the iterates are stored sparsely in either mode")
     if args.aln_format == "auto":
         detect_format(args)
-    unsupported = [("--correct_nrounds", args.correct_nrounds), ("--ul", args.ul), ("--gfa", args.gfa)]
+    if args.correct_nrounds and args.ul:
+        args.ul = None
+        logger.warning("Ultra-long data are not supported now when assembly correction is enabled")
+    unsupported = [("--ul", args.ul), ("--gfa", args.gfa)]
     for flag, val in unsupported:
         if val:
             raise NotImplementedError("haphic_b200: {} is not supported (out of the hot-path scope)".format(flag))
@@ -1283,19 +1287,32 @@ def run(args, log_file=None):
 
     fa_dict = parse_fasta(args.fasta, RE=args.RE)
     pos_int_type, dist_int_type = determine_int_type(fa_dict)
+    from . import hicio
+
+    def read_alignments(names, inter_only):
+        name_index = hicio.NameIndex(names)
+        if args.aln_format == "bam":
+            return hicio.bam_batches(args.alignments, name_index, inter_only=inter_only, logger=logger, threads=args.threads)
+        return hicio.pairs_batches(args.alignments, args.aln_format, name_index, inter_only=inter_only, threads=args.threads)
+
+    corrected = None
+    if args.correct_nrounds:
+        # one read of all read1 pairs serves both passes of the reference (1300-1398 and 2835-2851): the batches stay on the
+        # host, the same-contig ones feed the coverage, and the remapped batches are the second pass.  alignments.bed is
+        # written during this read, with the original names and coordinates, as the reference's second pass writes it.
+        from . import correct
+        logger.info("Parsing input {} file for contig correction...".format("BAM" if args.aln_format == "bam" else "pairs"))
+        corrected, _ = correct.run_correction(_context(), fa_dict, read_alignments(list(fa_dict), False), args)
     read_depth_dict = dict()
     whitelist = set()
     args.whitelist = whitelist
     _, bin_set, bin_size, frag_len_dict, Nx_frag_set, RE_site_dict, split_ctg_set = stat_fragments(
         fa_dict, args.RE, read_depth_dict, whitelist, nchrs=args.nchrs, flank=args.flank, Nx=args.Nx, bin_size=args.bin_size)
-    from . import hicio
     names = list(fa_dict.keys())
-    name_index = hicio.NameIndex(names)
-    inter_only = not split_ctg_set          # bins need the intra-contig pairs too (2849-2856)
-    if args.aln_format == "bam":
-        alignments = hicio.bam_batches(args.alignments, name_index, inter_only=inter_only, logger=logger, threads=args.threads)
+    if corrected is not None:
+        alignments = corrected
     else:
-        alignments = hicio.pairs_batches(args.alignments, args.aln_format, name_index, inter_only=inter_only, threads=args.threads)
+        alignments = read_alignments(names, inter_only=not split_ctg_set)      # bins need the intra-contig pairs too (2849-2856)
 
     # Two ways through the host side.  With --remove_allelic_links / --remove_concentrated_links the link dicts are
     # edited on the host, so they are built as the reference's Python objects.  Otherwise nothing on the host needs

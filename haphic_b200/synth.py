@@ -185,3 +185,64 @@ def write_pairs(asm: Assembly, pairs: np.ndarray, path: str) -> None:
         f.write("## pairs format v1.0\n#columns: readID chr1 pos1 chr2 pos2 strand1 strand2\n")
         for r, (a, pa, b, pb) in enumerate(pairs.tolist()):
             f.write("r{}\t{}\t{}\t{}\t{}\t+\t-\n".format(r, names[a], pa + 1, names[b], pb + 1))
+
+
+@dataclasses.dataclass
+class Misjoined:
+    asm: Assembly          # the misjoined assembly (chrom / start / ori of a joined contig are its first member's)
+    pairs: np.ndarray      # int32 [P, 4] the records re-expressed on it
+    junctions: dict        # name of a joined contig -> 0-based positions where one member ends and the next begins
+
+
+def make_misjoined(asm: Assembly, pairs, frac: float = 0.01, seed: int = 12345, prefix: str = "Mis") -> Misjoined:
+    """Join about ``frac * asm.n`` groups of 2 to 5 contigs, each from a different chromosome, end to end into chimeric
+    contigs ``{prefix}{k}``, and re-express the records on the result.  A joined contig takes the place of its first
+    member in FASTA order; the other contigs keep their names and order."""
+    rng = np.random.default_rng(seed)
+    pairs = np.asarray(pairs)
+    by_chrom = [list(rng.permutation(np.nonzero(asm.chrom == c)[0])) for c in range(asm.nchr)]
+    n_groups = max(1, int(round(frac * asm.n)))
+    groups = []
+    for _ in range(n_groups):
+        size = int(rng.integers(2, 6))
+        chroms = [c for c in rng.permutation(asm.nchr).tolist() if by_chrom[c]][:size]
+        if len(chroms) < 2:
+            break
+        groups.append([int(by_chrom[c].pop()) for c in chroms])
+    first_of = {g[0]: k for k, g in enumerate(groups)}
+    member = {c: k for k, g in enumerate(groups) for c in g}
+    names, lengths, chrom, start, ori = [], [], [], [], []
+    new_id = np.empty(asm.n, np.int64)
+    shift = np.zeros(asm.n, np.int64)
+    junctions = {}
+    for c in range(asm.n):
+        if c in member and c not in first_of:
+            continue
+        i = len(names)
+        if c in first_of:
+            g = groups[first_of[c]]
+            name = "{}{}".format(prefix, first_of[c] + 1)
+            p, cuts = 0, []
+            for m in g:
+                new_id[m], shift[m] = i, p
+                p += int(asm.lengths[m])
+                cuts.append(p)
+            junctions[name] = cuts[:-1]
+            names.append(name)
+            lengths.append(p)
+        else:
+            new_id[c] = i
+            names.append(asm.names[c])
+            lengths.append(int(asm.lengths[c]))
+        chrom.append(int(asm.chrom[c]))
+        start.append(int(asm.start[c]))
+        ori.append(int(asm.ori[c]))
+    out = pairs.astype(np.int64)
+    for e in (0, 2):
+        ok = (out[:, e] >= 0) & (out[:, e] < asm.n)
+        c = out[ok, e]
+        out[ok, e + 1] += shift[c]
+        out[ok, e] = new_id[c]
+    mis = Assembly(names, np.asarray(lengths, np.int64), np.asarray(chrom, np.int32), np.asarray(start, np.int64),
+                   np.asarray(ori, np.int8), asm.chrom_len, asm.nchr)
+    return Misjoined(mis, out.astype(np.int32), junctions)

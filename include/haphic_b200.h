@@ -246,6 +246,49 @@ int hh_mcl_commit(hh_mcl* mc);
 int hh_mcl_set_block(hh_mcl* mc, int32_t col_lo, int32_t col_hi);
 int hh_mcl_destroy(hh_mcl* mc);
 
+/* ---- assembly correction (`--correct_nrounds`): correct_assembly, HapHiC_cluster.py:943-1297 ------------------------
+ * Coverage of a contig is int32 over len // res + 1 bins (1312); contig c owns bins [bin_off[c], bin_off[c+1]) of one array
+ * and every fragment split from it is a sub-range of those bins (the reference slices numpy views, 1158 / 1180).  The
+ * intra-contig read pairs are kept as links {bucket, lo, hi} (lo <= hi, 0-based); a bucket is an id the host gives to a key
+ * string of ctg_link_pos_dict (initially bucket = contig id).
+ *   hh_correct_create:  res = --correct_resolution.
+ *   hh_correct_add:     parse_pairs_for_correction / parse_bam_for_correction (1300-1398): records {id_a, pos_a, id_b, pos_b}
+ *     with id_a == id_b in [0, n_ctg) add 1 to the bins [lo // res, hi // res] and append a link; other records are ignored.
+ *     A same-contig position outside [0, contig length) is an error.  Not allowed after the first detect / split / fetch.
+ *   hh_correct_info / hh_correct_fetch: bin count, link count; coverage [n_bins], bin_off [n_ctg + 1] and links [n_links][3]
+ *     (host buffers, any may be NULL).  Dropped links keep their slot with bucket -1.
+ *   hh_correct_detect:  detect_break_points (943-1014) on the fragments seg_off[s] (first bin), seg_nbins[s], seg_len[s] (bp):
+ *     n_bp[s] breakpoints each, packed in fragment order into bp_bin / bp_cov (bin relative to the fragment, its coverage;
+ *     the breakpoint is bin * res) up to max_bp entries; *total_bp = their number.
+ *   hh_correct_detect_segments: the same on a caller's host coverage array (stateless).
+ *   hh_correct_split:   one non-last round of break_and_update_ctgs (1074-1121) for n_frag broken fragments: fragment f holds
+ *     the links of bucket frag_bucket[f] (-1: none) and starts at bin frag_off[f]; shift_pos[list_off[f] .. list_off[f+1])
+ *     is pos_shift_list (its breakpoints descending, then 0) and piece_bucket[] the bucket of the key pos_shift gives each
+ *     entry.  frag_zero[f] = 0 (one non-zero breakpoint): links whose closed span overlaps [bp, bp + res] leave the coverage.
+ *     The other links move to the bucket of their piece with shifted coordinates; links across pieces are dropped.
+ *   hh_correct_set_pieces / hh_correct_remap: convert_ctg of the second pass (1405-1411).  Contig c's pieces are
+ *     [piece_off[c], piece_off[c+1]) with ascending 0-based starts (the first 0) and their ids in the corrected fa_dict;
+ *     remap rewrites every {id, pos} in place to {piece id, pos - piece start}; ids outside [0, n_ctg) become -1. */
+typedef struct hh_correct hh_correct;
+int hh_correct_create(hh_ctx* ctx, int32_t n_ctg, const int64_t* ctg_len, int32_t res, hh_correct** out);
+int hh_correct_add(hh_correct* hc, const int32_t* rec, int64_t n_rec, int mem);
+int hh_correct_info(hh_correct* hc, int64_t* n_bins, int64_t* n_links);
+int hh_correct_fetch(hh_correct* hc, int32_t* cov, int64_t* bin_off, int32_t* links);
+int hh_correct_detect(hh_correct* hc, int32_t n_seg, const int64_t* seg_off, const int32_t* seg_nbins, const int64_t* seg_len,
+                      double median_cov_ratio, double region_len_ratio, int64_t min_region_cutoff, int32_t* n_bp,
+                      int32_t* bp_bin, int32_t* bp_cov, int64_t max_bp, int64_t* total_bp);
+int hh_correct_detect_segments(hh_ctx* ctx, const int32_t* cov, int64_t n_cov, int32_t res, int32_t n_seg,
+                               const int64_t* seg_off, const int32_t* seg_nbins, const int64_t* seg_len,
+                               double median_cov_ratio, double region_len_ratio, int64_t min_region_cutoff, int32_t* n_bp,
+                               int32_t* bp_bin, int32_t* bp_cov, int64_t max_bp, int64_t* total_bp);
+int hh_correct_split(hh_correct* hc, int32_t n_frag, const int32_t* frag_bucket, const int64_t* frag_off,
+                     const uint8_t* frag_zero, const int32_t* list_off, const int32_t* shift_pos, const int32_t* piece_bucket,
+                     int32_t n_buckets);
+int hh_correct_set_pieces(hh_correct* hc, int32_t n_piece, const int32_t* piece_off, const int32_t* piece_start,
+                          const int32_t* piece_id);
+int hh_correct_remap(hh_correct* hc, int32_t* rec, int64_t n_rec, int mem);
+int hh_correct_destroy(hh_correct* hc);
+
 /* ---- host-side I/O around the path (native, no CUDA) ------------------------------------------------
  * .pairs / .pairs.gz reader: pairs_generator / pairs_generator_inter_ctgs, HapHiC_cluster.py:1539-1583.  Skips blank
  * and '#' lines, takes `cols[1], int(cols[2])-1, cols[3], int(cols[4])-1`, writes the two BED lines per pair
